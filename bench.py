@@ -3,6 +3,8 @@
 
     python bench.py --gpus N --steps K --warmup W            # this engine (B200)
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU path (oracle port)
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's S, b, g_cam,
+                                                             # cost and gradient as DIR/*.npy
 
 The metric is BASELINE.json's: observations/s through residual + analytic Jacobian + Schur
 accumulation (`value`, `e2e`), with the BA time-to-converge on the same data in `ba_converge`.
@@ -302,16 +304,22 @@ def local_scene(ctx, cams, frames, scaling):
     return sc, uvs, x0
 
 
-def timed_steps(ctx, prob, d_x, steps, warmup, sampler_index=None):
+def timed_steps(ctx, prob, d_x, steps, warmup, sampler_index=None, keep_outputs=False):
     """`warmup` untimed + `steps` timed passes of residual + Jacobian + Schur with everything resident
     in HBM; CUDA events on the problem's stream, barrier + synchronize on both sides, max over ranks.
-    Returns (ms total, per-kernel ms per step [K2p, K2c, SYRK, finalize + all-reduce], launches, clocks)."""
+    Returns (ms total, per-kernel ms per step [K2p, K2c, SYRK, finalize + all-reduce], launches, clocks,
+    outputs).  keep_outputs: the last timed pass also copies S, b, g_cam and the cost to the host (what a
+    caller of mcba_build_reduced receives) and `outputs` holds them; otherwise it is None."""
     torch, lib, h = ctx.torch, ctx.lib, prob._h
     check, null = ctx.native.check, ctypes.c_void_p()
     loss = ctx.native.LOSSES[LOSS]
+    nc = 12 * prob.C
+    outputs = {"S": np.empty((nc, nc)), "b": np.empty(nc), "g_cam": np.empty(nc), "cost": np.empty(1)} if keep_outputs else None
+    no_out = [null] * 4
+    last_out = [a.ctypes.data_as(ctypes.c_void_p) for a in outputs.values()] if keep_outputs else no_out
 
-    def step():
-        check(lib.mcba_build_reduced(h, ctypes.c_void_p(d_x.data_ptr()), LAMBDA, loss, 1.0, null, null, null, null))
+    def step(out=no_out):
+        check(lib.mcba_build_reduced(h, ctypes.c_void_p(d_x.data_ptr()), LAMBDA, loss, 1.0, *out))
 
     for _ in range(warmup):
         step()
@@ -321,8 +329,8 @@ def timed_steps(ctx, prob, d_x, steps, warmup, sampler_index=None):
     ctx.barrier()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record(prob.stream)
-    for _ in range(steps):
-        step()
+    for i in range(steps):
+        step(last_out if i == steps - 1 else no_out)
     e1.record(prob.stream)
     if sampler is not None and hasattr(sampler, "poll_until"):
         sampler.poll_until(e1)
@@ -333,7 +341,7 @@ def timed_steps(ctx, prob, d_x, steps, warmup, sampler_index=None):
     kn = ctypes.c_int()
     check(lib.mcba_profile(h, 0, kms, ctypes.byref(kn)))
     per = [kms[i] / max(kn.value, 1) for i in range(4)]
-    return ms, per, prob.kernel_launches - launches0, clocks
+    return ms, per, prob.kernel_launches - launches0, clocks, outputs
 
 
 def multi_gpu_parity(ctx, prob, uvs_local, obj, x_local):
@@ -447,9 +455,12 @@ def api_converge(ctx, scene, repeats=3):
                     + ("; every rank uploads and solves only its frames" if ctx.world > 1 else "")}
 
 
-def measure_problem(ctx, cams, frames, scaling, steps, warmup, sampler=False, parity=False, converge=True, e2e=True):
+def measure_problem(ctx, cams, frames, scaling, steps, warmup, sampler=False, parity=False, converge=True, e2e=True,
+                    keep_outputs=False):
     """One workload end to end on every rank: sharded problem, optional multi-GPU parity, timed
-    device-resident steps, e2e through host buffers, LM time-to-converge."""
+    device-resident steps, e2e through host buffers, LM time-to-converge.  keep_outputs: out["outputs"]
+    holds what the last timed step computed (S, b, g_cam, cost, and the full gradient [g_cam | g_pose]
+    of this rank's frames)."""
     from multicam_calibration_b200.engine import BAProblem
     torch = ctx.torch
     sc, uvs, x0 = local_scene(ctx, cams, frames, scaling)
@@ -461,7 +472,11 @@ def measure_problem(ctx, cams, frames, scaling, steps, warmup, sampler=False, pa
         out["parity"] = multi_gpu_parity(ctx, prob, uvs, sc.objpoints, x0)
     with torch.cuda.device(ctx.local), torch.cuda.stream(prob.stream):
         d_x = torch.as_tensor(x0).cuda()
-        ms, per, launches, clocks = timed_steps(ctx, prob, d_x, steps, warmup, ctx.local if (sampler and ctx.rank == 0) else None)
+        ms, per, launches, clocks, outputs = timed_steps(ctx, prob, d_x, steps, warmup,
+                                                         ctx.local if (sampler and ctx.rank == 0) else None, keep_outputs)
+        if keep_outputs:   # the gradient of the last evaluation, before e2e / converge evaluate again
+            outputs["gradient"] = prob.gradient()
+            out["outputs"] = outputs
         out["ms"] = ctx.max_over_ranks([ms])[0]
         out["kernels_ms"] = per                      # rank 0's launches
         out["kernels_ms_max"] = ctx.max_over_ranks(per)
@@ -511,6 +526,26 @@ def roofline_block(m, frames_local, peaks, peak_kind, fp64_peak):
                           "peak_source": "DFMA loop timed in this run (mcba_measure_fp64_peak)"},
             "note": "the kernel does ~250 FP64 FMAs per 16-byte observation: it is bound by the FP64 "
                     "pipe (fp64_pipe.frac), not by HBM; frac is the HBM figure the contract asks for"}
+
+
+DUMP_LIMIT_BYTES = 63_000_000     # under 64 MB with room for the .npy headers
+
+
+def dump_outputs(path, outputs):
+    """Write each output as `path/<name>.npy` (float64), smallest first.  An output that does not fit in
+    what is left of DUMP_LIMIT_BYTES is replaced by a fixed, seeded sample of its entries, with their
+    flat indices in `<name>_index.npy`, so that two builds can be compared output for output."""
+    os.makedirs(path, exist_ok=True)
+    left = DUMP_LIMIT_BYTES
+    for name, a in sorted(outputs.items(), key=lambda kv: kv[1].size):
+        a = np.asarray(a, dtype=np.float64)
+        if a.nbytes > left:
+            idx = np.sort(np.random.default_rng(0).choice(a.size, left // 16, replace=False))
+            a = a.ravel()[idx]
+            np.save(os.path.join(path, name + "_index.npy"), idx.astype(np.float64))
+            left -= a.nbytes
+        np.save(os.path.join(path, name + ".npy"), a)
+        left -= a.nbytes
 
 
 def kernels_block(per):
@@ -680,7 +715,10 @@ def run_engine(args):
         frames = cfg["frames"] // cfg["quoted_gpus"]      # per GPU
     else:
         frames = cfg["frames"]                            # total
-    main = measure_problem(ctx, cams, frames, args.scaling, args.steps, args.warmup, sampler=True, parity=True)
+    main = measure_problem(ctx, cams, frames, args.scaling, args.steps, args.warmup, sampler=True, parity=True,
+                           keep_outputs=bool(args.dump_outputs))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, main.pop("outputs"))
 
     # ---- the public call: numpy arrays in, calibration out (N > 1: the 50k-frame problem sharded inside the call)
     import multicam_calibration_b200 as mcc
@@ -806,7 +844,14 @@ def main():
     ap.add_argument("--points", type=int, default=1_000_000, help="keypoints of the configs[4] extra")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="headline only: no strong / configs[3] / configs[4] / K1 blocks")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write what the last one computed (rank 0: S, b, g_cam, cost and the "
+                         "gradient [g_cam | g_pose] of its frames) as DIR/<name>.npy, float64, at most 64 MB in all")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "engine":
+        ap.error("--dump-outputs applies to the engine arm only")
     args.warmup = max(args.warmup, 3) if args.impl == "engine" else args.warmup
     out = _quiet_stdout()
     line = run_reference(args) if args.impl == "reference" else run_engine(args)

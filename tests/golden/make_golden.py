@@ -236,10 +236,13 @@ def gen_ba_cfg1(geo, ba):
     sparse Jacobian and a sparse direct solve (``oracle.sparse_gauss_newton_polish``); the stored
     ``optimality_tight`` (||J^T rho' f||_inf at x_tight, evaluated with the reference residuals) is
     its certificate."""
+    import hashlib
+    import json
     import time
     from oracle import np_oracle as orc
     from multicam_calibration_b200.synthetic import make_scene
-    sc = make_scene(6, 500, sigma=0.3, seed=0)
+    scene = dict(n_cameras=6, n_frames=500, sigma=0.3, seed=0)
+    sc = make_scene(**scene)
     args = sc.init_args()
     np.random.seed(0)
     buf = io.StringIO()
@@ -256,7 +259,11 @@ def gen_ba_cfg1(geo, ba):
           f"after {len(trace)} Gauss-Newton steps")
     assert g_t < 1e-6
     x0 = ba.serialize_params(args[1], args[2], args[4][use_d])
-    return dict(versions=_versions(), uvs=sc.uvs, objpoints=sc.objpoints, init_cams=sc.init_cams,
+    # the 1.7 MB observation array is not stored: tests/conftest.py regenerates it from `scene` and
+    # checks it against `uvs_sha256`
+    return dict(versions=_versions(), scene=np.array(json.dumps(scene)),
+                uvs_sha256=np.array(hashlib.sha256(np.ascontiguousarray(sc.uvs).tobytes()).hexdigest()),
+                objpoints=sc.objpoints, init_cams=sc.init_cams,
                 init_poses=sc.init_poses, use_frames=use_d, x0=x0, msg_default=np.array(buf.getvalue()),
                 x_default=r_d.x, cost_default=r_d.cost, rms_default=rms(r_d.x), nfev_default=r_d.nfev,
                 njev_default=r_d.njev, status_default=r_d.status, optimality_default=r_d.optimality,
