@@ -279,6 +279,29 @@ int mcba_download(int device, void* cuda_stream, void* h_dst, const void* d_src,
 /* Number of kernels this handle has launched (bench.py gpu_launches). */
 int64_t mcba_kernel_launches(mcba_handle* h);
 
+/* Kernel variants the handle's evaluation and solve take for its shape and observations (the launch
+ * heuristics' choices, for tests that must show which branches they reached).  out[n] receives, at the
+ * indices below: K2p warps per CTA and grid; K2c mode (0 general, 1 staged ring, 2 streamed pair),
+ * warps of the streamed pair (0 otherwise) and its per-CTA partial count; SYRK warps, CTA rows (gy) and
+ * the block count of its compiled tile list (0: listed at run time); the reduced solve (0 cuSOLVER,
+ * 3 / 8 / 19 register tiles per warp, 119 = 19 tiles with the trailing ones in shared memory); frame
+ * tiles; back-substitution grid; C; then the live (tile, camera) units of every camera (C entries).
+ * n must be at least MCBA_PLAN_UNITS + C.  Synchronises the handle's stream. */
+#define MCBA_PLAN_K2P_WARPS 0
+#define MCBA_PLAN_K2P_GRID 1
+#define MCBA_PLAN_K2C_MODE 2
+#define MCBA_PLAN_K2C_WARPS 3
+#define MCBA_PLAN_K2C_PARTS 4
+#define MCBA_PLAN_SYRK_WARPS 5
+#define MCBA_PLAN_SYRK_GY 6
+#define MCBA_PLAN_SYRK_STATIC_NB 7
+#define MCBA_PLAN_SOLVE 8
+#define MCBA_PLAN_TILES 9
+#define MCBA_PLAN_BACKSUB_GRID 10
+#define MCBA_PLAN_CAMERAS 11
+#define MCBA_PLAN_UNITS 12
+int mcba_plan_info(mcba_handle* h, int64_t* out, int n);
+
 #ifdef __cplusplus
 }
 #endif

@@ -16,6 +16,12 @@ ERR_NONFINITE = -4
 LOSSES = {"linear": 0, "soft_l1": 1, "soft_l1_irls": 0x101}
 HESSIANS = {"auto": 0, "triggs": 1, "irls": 2}
 
+# mcba_plan_info: indices of the launch choices (include/mcba.h MCBA_PLAN_*); the live units per camera follow
+PLAN_FIELDS = ("k2p_warps", "k2p_grid", "k2c_mode", "k2c_warps", "k2c_parts", "syrk_warps", "syrk_gy",
+               "syrk_static_nb", "solve", "tiles", "backsub_grid", "cameras")
+K2C_MODES = {0: "general", 1: "ring", 2: "stream"}
+SOLVE_TIERS = {0: "cusolver", 3: "regs3", 8: "regs8", 19: "regs19", 119: "smem19"}
+
 ITER_CALLBACK = ctypes.CFUNCTYPE(None, ctypes.c_void_p, ctypes.c_int, ctypes.c_int, ctypes.c_double,
                                  ctypes.c_double, ctypes.c_double, ctypes.c_double)
 
@@ -77,6 +83,7 @@ _SIGNATURES = {
     "mcba_undistort_points": (_I, [_I, _P, _P, _L, _P, _P, _P]),
     "mcba_triangulate": (_I, [_I, _P, _P, _I, _L, _P, _P, _P, _P]),
     "mcba_kernel_launches": (_L, [_P]),
+    "mcba_plan_info": (_I, [_P, ctypes.POINTER(_L), _I]),
     "mcba_profile": (_I, [_P, _I, ctypes.POINTER(_D), ctypes.POINTER(_I)]),
     "mcba_measure_fp64_peak": (_I, [_I, ctypes.POINTER(_D)]),
     "mcba_select_frames": (_I, [_I, _P, _P, _I, _L, _I, _P, _P, _D, _P, ctypes.POINTER(_D)]),

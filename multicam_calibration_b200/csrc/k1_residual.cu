@@ -213,7 +213,11 @@ int launch_tile_observations(mcba_handle* h) {
   const int grid = (int)(units < 148 * 8 ? units : 148 * 8);
   unsigned long long* n_scalars = reinterpret_cast<unsigned long long*>(h->d_unit_count + 96);
   MCBA_CUDA(cudaMemsetAsync(n_scalars, 0, sizeof(unsigned long long), h->stream));
-  tile_observations_kernel<<<grid, 256, sizeof(double2) * kTile * (L.N + 1), h->stream>>>(
+  // 16 * 32 * (N + 1) bytes: above the 48 KB default from 96 corners on (mcba_create rejects boards whose
+  // transpose does not fit the device's opt-in limit)
+  const size_t tile_smem = tile_observations_smem(L.N);
+  MCBA_CUDA(set_dynamic_smem((const void*)tile_observations_kernel, tile_smem));
+  tile_observations_kernel<<<grid, 256, tile_smem, h->stream>>>(
       reinterpret_cast<const double2*>(h->d_obs_ref), h->d_obs_tiled, h->d_perm, L.C, L.F, L.N, units, n_scalars);
   build_units_kernel<<<L.C, 256, 0, h->stream>>>(h->d_active, L.nTiles, h->d_units, h->d_unit_count);
   group_prefix_kernel<<<1, 32, 0, h->stream>>>(h->d_unit_count, L.C, h->prod_warps, h->d_unit_count + 32);
@@ -360,7 +364,9 @@ __global__ void __launch_bounds__(256, MCBA_K1_CTAS) residual_chunks_kernel(cons
   const long long nUnits = (long long)C * nBlk;
   const long long gw = (long long)blockIdx.x * nWarps + warp, stride = (long long)gridDim.x * nWarps;
   // slot -> row within the chunk: i / N for i < 32 N <= 2^16 N ... exact for i * N < 2^32 with a 32-bit reciprocal
+  // (N = 1: the reciprocal 2^32 does not fit in 32 bits, and the row is the slot itself)
   const unsigned inv_n = (unsigned)((0x100000000ull + (unsigned)N - 1) / (unsigned)N);
+  auto row_of = [&](int i) { return N == 1 ? i : (int)__umulhi((unsigned)i, inv_n); };
   const unsigned lt = (1u << lane) - 1u;
   for (long long u = gw; u < nUnits; u += stride) {
     const int c = (int)(u / nBlk);
@@ -411,7 +417,7 @@ __global__ void __launch_bounds__(256, MCBA_K1_CTAS) residual_chunks_kernel(cons
         const int i = i0 + g * 32 + lane;
         o[g] = make_double2(qnan, qnan);
         if (kCompact && (!kChecked || i < total)) {
-          const int q = (int)__umulhi((unsigned)i, inv_n);
+          const int q = row_of(i);
           o[g] = ref[base + (s_rk[q] - q) * N + i];
         }
       }
@@ -422,7 +428,7 @@ __global__ void __launch_bounds__(256, MCBA_K1_CTAS) residual_chunks_kernel(cons
         bool fu = false, fv = false;
         double ru = 0.0, rv = 0.0;
         if (!kChecked || i < total) {
-          const int q = (int)__umulhi((unsigned)i, inv_n);   // rank of the slot's row among the live rows
+          const int q = row_of(i);   // rank of the slot's row among the live rows
           const int n = i - q * N;
           const double2* t = reinterpret_cast<const double2*>(s_T + q * 12);
           const double2 t0 = t[0], t1 = t[1], t2 = t[2], t3 = t[3], t4 = t[4], t5 = t[5];

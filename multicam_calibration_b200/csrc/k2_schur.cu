@@ -330,6 +330,23 @@ int syrk_grid(int nc, long long F, int n_sm) {
   return (int)(tiles < n_sm ? tiles : n_sm);
 }
 
+// Block count of the compiled tile list the SYRK uses for a 12C-wide system, 0 when the tiles are listed at
+// run time (more than one CTA row, no compiled list for this width, or MCBA_SYRK_RUNTIME set).
+static int syrk_static_nb(const SyrkConfig& c, int nc) {
+  static const bool no_static = getenv("MCBA_SYRK_RUNTIME") != nullptr;   // A/B: run-time tile lists
+  const int nb8 = (nc + 7) / 8;
+  if (c.gy != 1 || no_static) return 0;
+  if (c.warps == 8) return (nb8 == 3 || nb8 == 5 || nb8 == 6 || nb8 == 8 || nb8 == 9 || nb8 == 12) ? nb8 : 0;
+  return (nb8 == 18 || nb8 == 24) ? nb8 : 0;
+}
+
+void syrk_plan(int nc, int* warps, int* gy, int* static_nb) {
+  const SyrkConfig c = syrk_config(nc);
+  *warps = c.warps;
+  *gy = c.gy;
+  *static_nb = syrk_static_nb(c, nc);
+}
+
 int launch_k2_syrk(mcba_handle* h) {
   const Layout& L = h->L;
   const SyrkConfig c = syrk_config(L.nc);
@@ -339,13 +356,12 @@ int launch_k2_syrk(mcba_handle* h) {
   p.nTiles = (int)L.nTiles;
   p.KW = c.KW;
   p.part = h->d_partSyrk;
-  static const bool no_static = getenv("MCBA_SYRK_RUNTIME") != nullptr;   // A/B: run-time tile lists
 #define MCBA_SYRK(W, NB)                                                                                          \
   do {                                                                                                            \
     MCBA_CUDA(set_dynamic_smem((const void*)k2_syrk_kernel<W, NB>, c.smem)); \
     k2_syrk_kernel<W, NB><<<dim3(h->grid_syrk, c.gy), (W + 1) * 32, c.smem, h->stream>>>(p);                      \
   } while (0)
-  const int nb = (c.gy == 1 && !no_static) ? p.nb8 : 0;
+  const int nb = syrk_static_nb(c, L.nc);
   if (c.warps == 8) {
     switch (nb) {
       case 3: MCBA_SYRK(8, 3); break;    // 2 cameras

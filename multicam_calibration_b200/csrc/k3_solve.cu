@@ -298,25 +298,35 @@ bool solve_uses_library(int nc) {
   return force || nc > kSolveMaxN;
 }
 
+// Which solve runs for a 12C-wide system: kSolveTier* (mcba_plan_info).
+int solve_tier(int nc) {
+  if (solve_uses_library(nc)) return kSolveTierLibrary;
+  const int n1p = (nc + 1 + 7) & ~7;
+  const int nb = n1p / 8, per_warp = ((nb - 1) * nb / 2 + kSolveWarps - 1) / kSolveWarps;
+  static const bool wide_in_registers = getenv("MCBA_SOLVE_WIDE_REGS") != nullptr;   // A/B: the spilling variant
+  if (per_warp <= 3) return kSolveTierRegs3;
+  if (per_warp <= 8) return kSolveTierRegs8;
+  return wide_in_registers ? kSolveTierRegs19 : kSolveTierSmem19;
+}
+
 int solve_reduced(mcba_handle* h, double lambda) {
   const Layout& L = h->L;
   const int nc = L.nc;
-  if (!solve_uses_library(nc)) {
+  const int tier = solve_tier(nc);
+  if (tier != kSolveTierLibrary) {
     SolveParams p;
     p.red = h->d_red; p.offS = L.offS; p.offB = L.offB; p.offDiag = L.offDiag; p.nc = nc; p.lambda = lambda;
     p.D2cam = h->d_D2cam; p.dcam = h->d_dcam; p.info = h->d_info;
     const int n1p = (nc + 1 + 7) & ~7;
     const size_t smem = sizeof(double) * (size_t)n1p * (n1p + 1) / 2;
-    const int nb = n1p / 8, per_warp = ((nb - 1) * nb / 2 + kSolveWarps - 1) / kSolveWarps;
 #define MCBA_SOLVE(...)                                                                                                    \
   do {                                                                                                                     \
     MCBA_CUDA(set_dynamic_smem((const void*)solve_reduced_kernel<__VA_ARGS__>, smem)); \
     solve_reduced_kernel<__VA_ARGS__><<<1, kSolveThreads, smem, h->stream>>>(p);                                           \
   } while (0)
-    static const bool wide_in_registers = getenv("MCBA_SOLVE_WIDE_REGS") != nullptr;   // A/B: the spilling variant
-    if (per_warp <= 3) MCBA_SOLVE(3);
-    else if (per_warp <= 8) MCBA_SOLVE(8);
-    else if (wide_in_registers) MCBA_SOLVE(19);
+    if (tier == kSolveTierRegs3) MCBA_SOLVE(3);
+    else if (tier == kSolveTierRegs8) MCBA_SOLVE(8);
+    else if (tier == kSolveTierRegs19) MCBA_SOLVE(19);
     else MCBA_SOLVE(19, true);
 #undef MCBA_SOLVE
 #ifdef MCBA_SOLVE_TIMING

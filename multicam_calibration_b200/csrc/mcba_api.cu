@@ -331,6 +331,13 @@ static int create_impl(mcba_handle* h, int C, int64_t F, int N, int device) {
   L.redLen = L.offRank + kMaxRanks;
   cudaDeviceProp prop;
   MCBA_CUDA(cudaGetDeviceProperties(&prop, device));
+  if (tile_observations_smem(N) > prop.sharedMemPerBlockOptin) {
+    set_error("mcba_create: a board of " + std::to_string(N) + " points needs " + std::to_string(tile_observations_smem(N)) +
+              " bytes of shared memory to tile its observations; this device allows " +
+              std::to_string(prop.sharedMemPerBlockOptin) + " per block (at most " +
+              std::to_string(prop.sharedMemPerBlockOptin / (sizeof(double2) * kTile) - 1) + " points)");
+    return MCBA_ERR_ARG;
+  }
   h->n_sm = prop.multiProcessorCount;
   MCBA_CUDA(cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking));
   h->grid_frames = k2_producer_grid(L, h->n_sm, &h->prod_warps);
@@ -1068,6 +1075,36 @@ int mcba_comm_init(mcba_handle* h, const void* id128, int rank, int nranks) {
 }
 
 int64_t mcba_kernel_launches(mcba_handle* h) { return h ? h->launches : 0; }
+
+int mcba_plan_info(mcba_handle* h, int64_t* out, int n) {
+  int rc = need_obs(h);
+  if (rc) return rc;
+  const Layout& L = h->L;
+  const int need = MCBA_PLAN_UNITS + L.C;
+  if (!out || n < need) {
+    set_error("mcba_plan_info: out needs " + std::to_string(need) + " entries");
+    return MCBA_ERR_ARG;
+  }
+  int units[32];
+  MCBA_CUDA(cudaMemcpyAsync(units, h->d_unit_count, sizeof(int) * L.C, cudaMemcpyDeviceToHost, h->stream));
+  MCBA_CUDA(cudaStreamSynchronize(h->stream));
+  int sw = 0, gy = 0, nb = 0;
+  syrk_plan(L.nc, &sw, &gy, &nb);
+  out[MCBA_PLAN_K2P_WARPS] = h->prod_warps;
+  out[MCBA_PLAN_K2P_GRID] = h->grid_frames;
+  out[MCBA_PLAN_K2C_MODE] = h->k2c_mode;
+  out[MCBA_PLAN_K2C_WARPS] = h->k2c_mode == 2 ? k2c_stream_warps(L.C) : 0;
+  out[MCBA_PLAN_K2C_PARTS] = h->n_part_c;
+  out[MCBA_PLAN_SYRK_WARPS] = sw;
+  out[MCBA_PLAN_SYRK_GY] = gy;
+  out[MCBA_PLAN_SYRK_STATIC_NB] = nb;
+  out[MCBA_PLAN_SOLVE] = solve_tier(L.nc);
+  out[MCBA_PLAN_TILES] = L.nTiles;
+  out[MCBA_PLAN_BACKSUB_GRID] = h->grid_back;
+  out[MCBA_PLAN_CAMERAS] = L.C;
+  for (int c = 0; c < L.C; ++c) out[MCBA_PLAN_UNITS + c] = units[c];
+  return MCBA_OK;
+}
 
 int mcba_profile(mcba_handle* h, int enable, double* ms_out, int* n_out) {
   if (!h) return MCBA_ERR_ARG;

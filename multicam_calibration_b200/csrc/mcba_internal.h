@@ -181,6 +181,14 @@ int launch_k2_consumer(mcba_handle* h, const double* x, double lambda);
 int launch_k2_gradient(mcba_handle* h, const double* x);   // pose gradient only (closing evaluation)
 int k2_producer_grid(const mcba::Layout& L, int n_sm, int* warps);
 int k2_consumer_parts(const mcba::Layout& L, int n_sm, int* mode);
+int k2c_stream_warps(int C);
+// SYRK CTA width (warps), CTA rows (gy) and the block count of the compiled tile list (0: run-time list)
+void syrk_plan(int nc, int* warps, int* gy, int* static_nb);
+// solve of the reduced system: tiles per warp of the one-CTA kernel, or the library
+enum SolveTier : int { kSolveTierLibrary = 0, kSolveTierRegs3 = 3, kSolveTierRegs8 = 8, kSolveTierRegs19 = 19, kSolveTierSmem19 = 119 };
+int solve_tier(int nc);
+// dynamic shared memory of the observation transpose (k1_residual.cu): [32 frames][N + 1] corners
+inline size_t tile_observations_smem(int N) { return sizeof(double2) * kTile * ((size_t)N + 1); }
 int launch_k2_syrk(mcba_handle* h);
 int syrk_grid(int nc, long long F, int n_sm);
 int launch_finalize(mcba_handle* h, bool exchange);   // exchange: sum over ranks inside the kernel (peer memory)

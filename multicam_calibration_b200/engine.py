@@ -267,6 +267,20 @@ class BAProblem:
     def kernel_launches(self):
         return int(self.lib.mcba_kernel_launches(self._h))
 
+    @_on_stream
+    def plan_info(self):
+        """Kernel variants this problem's evaluation and solve take (``mcba_plan_info``): a dict of
+        ``_native.PLAN_FIELDS`` with ``k2c_mode`` and ``solve`` named, plus ``units``, the live
+        (tile, camera) units of every camera."""
+        n = len(_native.PLAN_FIELDS) + self.C
+        out = (ctypes.c_int64 * n)()
+        check(self.lib.mcba_plan_info(self._h, out, n))
+        info = dict(zip(_native.PLAN_FIELDS, (int(v) for v in out)))
+        info["k2c_mode"] = _native.K2C_MODES[info["k2c_mode"]]
+        info["solve"] = _native.SOLVE_TIERS[info["solve"]]
+        info["units"] = [int(v) for v in out[len(_native.PLAN_FIELDS):]]
+        return info
+
     # ------------------------------------------------------------------ per-call operators
     @_on_stream
     def residuals(self, params):

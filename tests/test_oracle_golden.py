@@ -219,3 +219,65 @@ def test_transformation_vectors_match_reference():
     g = load_golden("init")
     np.testing.assert_allclose(orc.rodrigues_inv(g["R"]), g["R_vec"], rtol=0, atol=1e-15)
     np.testing.assert_allclose(orc.transformation_vector(g["T"]), g["T_vec"], rtol=0, atol=1e-15)
+
+
+# ------------------------------------------------------------------ blockwise reference at scale (oracle/blockwise.py)
+def _pinning_scene(lam):
+    """4 cameras x 30 frames with every irregular input the blockwise reference must handle: camera 2 sees
+    nothing, frames 3 and 17 are seen by no camera, a few corners are half observed (u without v), two
+    frames are gross outliers (shifted by 1e3 / 1e5 px) and one pose has rotation norm 0.  At lam = 0 the
+    outlier frames are left unobserved instead: their pose blocks (robust weights down to the EPS clamp)
+    are too ill-conditioned for two elimination orders to agree to 1e-12 without damping."""
+    from multicam_calibration_b200.synthetic import make_scene
+    sc = make_scene(4, 30, sigma=0.4, p_missing_view=0.2, p_missing_corner=0.05, seed=12)
+    uvs = sc.uvs.copy()
+    uvs[2] = np.nan
+    uvs[:, [3, 17]] = np.nan
+    uvs[0, 5, 3, 1] = np.nan
+    uvs[1, 6, 10, 0] = np.nan
+    uvs[3, 8, 0, 1] = np.nan
+    uvs[:, 11] += 1e3
+    uvs[:, 23, :, 0] += 1e5
+    if lam == 0.0:
+        uvs[:, [11, 23]] = np.nan
+    x = sc.x0()
+    x[48 + 6 * 9:48 + 6 * 9 + 3] = 0.0
+    return uvs, sc.objpoints, x
+
+
+@pytest.mark.parametrize("loss,hessian,f_scale,lam", [
+    ("linear", "triggs", 1.0, 0.0), ("linear", "triggs", 0.25, 1e-2), ("soft_l1", "triggs", 1.0, 1e-2),
+    ("soft_l1", "triggs", 0.25, 0.0), ("soft_l1", "triggs", 4.0, 1e-2), ("soft_l1", "irls", 0.25, 1e-2),
+    ("soft_l1", "irls", 4.0, 0.0)])
+def test_blockwise_reference_matches_the_dense_oracle(loss, hessian, f_scale, lam):
+    """oracle.blockwise (what the GPU tests at 50,000 frames compare the kernels with) against the dense
+    normal equations of np_oracle: S, b, both gradients and the cost to 1e-12, the damped step to 1e-10.
+    Chunks of 7 frames (the last one short) run the chunked accumulation."""
+    from oracle import blockwise
+    uvs, obj, x = _pinning_scene(lam)
+    C, F = uvs.shape[:2]
+    nc = 12 * C
+    ev = blockwise.BlockwiseEvaluation(x, uvs, obj, lam=lam, loss=loss, f_scale=f_scale, hessian=hessian, chunk=7)
+    assert np.array_equal(ev.empty, np.isnan(uvs).all((0, 2, 3))) and ev.empty[[3, 17]].all()
+    H, g, cost = orc.normal_equations(x, uvs, obj, loss=loss, f_scale=f_scale, hessian=hessian)
+    D2 = np.diag(H).copy()
+    D2[D2 == 0.0] = 1.0
+    if lam == 0.0:   # frames nobody sees contribute nothing; the dense elimination would invert their zero blocks
+        keep = np.r_[np.arange(nc), nc + (np.nonzero(~ev.empty)[0][:, None] * 6 + np.arange(6)).ravel()]
+        S_o, b_o = orc.reduced_camera_system(H[np.ix_(keep, keep)], g[keep], C, 0.0)
+    else:
+        S_o, b_o = orc.reduced_camera_system(H, g, C, lam, np.r_[np.zeros(nc), D2[nc:]])
+    assert ev.cost == pytest.approx(cost, rel=1e-12)
+    assert np.abs(ev.g_cam - g[:nc]).max() <= 1e-12 * np.abs(g).max()
+    assert np.abs(ev.g_pose.ravel() - g[nc:]).max() <= 1e-12 * np.abs(g).max()
+    assert np.abs(ev.S - S_o).max() <= 1e-12 * np.abs(S_o).max()
+    assert np.abs(ev.b - b_o).max() <= 1e-12 * np.abs(b_o).max()
+    assert np.array_equal(ev.diag_U, np.diag(H)[:nc]) or np.abs(ev.diag_U - np.diag(H)[:nc]).max() <= 1e-12 * np.diag(H).max()
+    assert (ev.diag_U[24:36] == 0).all() and (ev.g_pose[ev.empty] == 0).all()
+    if lam:
+        step = ev.step()
+        step_o = orc.lm_step(H, g, C, lam, D2)
+        assert np.abs(step - step_o).max() <= 1e-10 * np.abs(step_o).max()
+        assert (step[nc:].reshape(F, 6)[ev.empty] == 0).all()
+        S2, b2, gc2, gp2, c2 = blockwise.reduced_camera_system_blockwise(x, uvs, obj, lam, loss, f_scale, hessian)
+        assert np.abs(S2 - ev.S).max() <= 1e-13 * np.abs(S_o).max() and c2 == pytest.approx(ev.cost, rel=1e-14)
