@@ -144,6 +144,28 @@ int mcba_solve_step(mcba_handle* h, const double* d_x, double lambda, double* d_
 int mcba_lm_run(mcba_handle* h, double* d_x, const mcba_options* opt, mcba_result* res,
                 double* d_grad);
 
+/* Covariance of the calibration at d_x: the block inverse of the Gauss-Newton matrix H = J~^T J~, J~ the residual
+ * Jacobian row-scaled as scipy's scale_for_robust_loss_function does (weights max(rho' + 2 rho'' z, EPS) for
+ * soft_l1, whatever a solve's hessian option was; lambda = 0), times the residual variance s^2.  The 6 extrinsic
+ * parameters of reference_camera are held fixed (the gauge).  One evaluation (K2p, K2c, SYRK, finalize), the
+ * gauge-fixed inverse of the reduced camera system and one pass over the frames.
+ *   h_cam_cov   (12C x 12C, host, row major, caller's parameter basis): s^2 S^-1; exactly 0 on the reference
+ *               camera's extrinsic rows / columns, NaN on the rows / columns of cameras without observations.
+ *   d_pose_cov  (F, 6, 6, device, may be NULL): s^2 (V^-1 + V^-1 W^T S^-1 W V^-1) per frame, [rvec | tvec];
+ *               NaN for frames without observations.
+ *   sigma2      > 0: s^2 = sigma2; <= 0: s^2 = 2 cost / (m - p), m finite scalar residuals,
+ *               p = 12 (observed cameras) + 6 (observed frames) - 6.
+ *   h_stats     (host, may be NULL) [9]: s^2, m - p, m, cost, frames without observations, smallest relative
+ *               Cholesky pivot of the observed frames' pose blocks, then device ms of {evaluation + frame check,
+ *               camera inverse, pose pass}.
+ * Errors: MCBA_ERR_ARG for a bad loss / reference_camera, a reference camera without observations or m <= p
+ * (sigma2 <= 0); MCBA_ERR_NONFINITE for residuals that are not finite at d_x; MCBA_ERR_SOLVER when an observed
+ * frame's pose block or the Jacobi-scaled gauge-fixed camera system has a relative Cholesky pivot <= 1e-12.
+ * Single-rank handles only.  The running Marquardt scaling is left as it was; as after mcba_build_reduced, a
+ * following mcba_solve_step / mcba_gradient refer to this call's (lambda = 0) evaluation. */
+int mcba_covariance(mcba_handle* h, const double* d_x, int loss, double f_scale, int reference_camera, double sigma2,
+                    double* h_cam_cov, double* d_pose_cov, double* h_stats);
+
 /* Gradient of 0.5*sum rho at the last evaluated point, [g_cam (12C) | g_pose (6F)] (device). */
 int mcba_gradient(mcba_handle* h, double* d_grad);
 

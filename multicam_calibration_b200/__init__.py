@@ -5,7 +5,8 @@
 reference builds with its star imports (``multicam_calibration/__init__.py:1-7``)
 for the two hot-path modules, plus the steps on either side of them: the rigid-transform part of
 ``calibration`` that produces bundle_adjust's initial guess (calibration.py:116-277), the
-reprojection-error check of its result (viz.py:70-210) and the calibration files (io.py:8-245).
+reprojection-error check of its result (viz.py:70-210) and the calibration files (io.py:8-245), and the
+covariance of a calibration (``calibration_covariance``: what a reference user derives from ``result.jac``).
 """
 from .geometry import (rodrigues, rodrigues_inv, rigid_transform_from_correspondences,
                        apply_rigid_transform, get_transformation_matrix, get_transformation_vector,
@@ -20,5 +21,6 @@ from .calibration import (estimate_pairwise_camera_transform, get_camera_spannin
 from .io import save_calibration, load_calibration
 from .viz import plot_residuals, reprojection_residuals
 from .engine import BAProblem, OptimizeResult
+from .covariance import calibration_covariance, CalibrationCovariance
 
 __version__ = "0.1.0"

@@ -12,6 +12,8 @@ LIB_PATH = os.path.join(_HERE, "libmcba.so")
 CSRC = os.path.join(_HERE, "csrc")
 
 MCBA_OK = 0
+ERR_ARG = -1
+ERR_SOLVER = -3
 ERR_NONFINITE = -4
 LOSSES = {"linear": 0, "soft_l1": 1, "soft_l1_irls": 0x101}
 HESSIANS = {"auto": 0, "triggs": 1, "irls": 2}
@@ -71,6 +73,7 @@ _SIGNATURES = {
     "mcba_build_reduced_host": (_I, [_P, _P, _P, _P, _D, _I, _D, _P, _P, _P]),
     "mcba_solve_step": (_I, [_P, _P, _D, _P]),
     "mcba_gradient": (_I, [_P, _P]),
+    "mcba_covariance": (_I, [_P, _P, _I, _D, _I, _D, _P, _P, _P]),
     "mcba_lm_run": (_I, [_P, _P, ctypes.POINTER(Options), ctypes.POINTER(Result), _P]),
     "mcba_comm_unique_id": (_I, [_P]),
     "mcba_comm_init": (_I, [_P, _P, _I, _I]),

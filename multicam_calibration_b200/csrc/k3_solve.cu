@@ -309,6 +309,22 @@ int solve_tier(int nc) {
   return wide_in_registers ? kSolveTierRegs19 : kSolveTierSmem19;
 }
 
+// cuSOLVER handle on the handle's stream and the potrf workspace of the 12C-wide solve, created on first use
+// (the common sizes never touch the library; the covariance's camera inverse does)
+int ensure_solver(mcba_handle* h) {
+  if (!h->solver) {
+    const int nc = h->L.nc;
+    if (cusolverDnCreate(&h->solver) != CUSOLVER_STATUS_SUCCESS) { set_error("cusolverDnCreate failed"); return MCBA_ERR_SOLVER; }
+    if (cusolverDnDpotrf_bufferSize(h->solver, CUBLAS_FILL_MODE_LOWER, nc, h->d_Sd, nc, &h->lwork) != CUSOLVER_STATUS_SUCCESS) {
+      set_error("cusolverDnDpotrf_bufferSize failed");
+      return MCBA_ERR_SOLVER;
+    }
+    MCBA_CUDA(cudaMalloc((void**)&h->d_work, sizeof(double) * (size_t)(h->lwork > 0 ? h->lwork : 1)));
+  }
+  cusolverDnSetStream(h->solver, h->stream);
+  return MCBA_OK;
+}
+
 int solve_reduced(mcba_handle* h, double lambda) {
   const Layout& L = h->L;
   const int nc = L.nc;
@@ -341,15 +357,8 @@ int solve_reduced(mcba_handle* h, double lambda) {
     MCBA_CUDA(cudaGetLastError());
     return MCBA_OK;
   }
-  if (!h->solver) {   // created on first use: the common sizes never touch the library
-    if (cusolverDnCreate(&h->solver) != CUSOLVER_STATUS_SUCCESS) { set_error("cusolverDnCreate failed"); return MCBA_ERR_SOLVER; }
-    if (cusolverDnDpotrf_bufferSize(h->solver, CUBLAS_FILL_MODE_LOWER, nc, h->d_Sd, nc, &h->lwork) != CUSOLVER_STATUS_SUCCESS) {
-      set_error("cusolverDnDpotrf_bufferSize failed");
-      return MCBA_ERR_SOLVER;
-    }
-    MCBA_CUDA(cudaMalloc((void**)&h->d_work, sizeof(double) * (size_t)(h->lwork > 0 ? h->lwork : 1)));
-  }
-  cusolverDnSetStream(h->solver, h->stream);
+  int rc = ensure_solver(h);
+  if (rc) return rc;
   damp_kernel<<<(nc * nc + 255) / 256, 256, 0, h->stream>>>(h->d_red, L.offS, L.offB, L.offDiag, nc, lambda,
                                                             h->d_D2cam, h->d_Sd, h->d_dcam);
   h->launches++;

@@ -854,6 +854,99 @@ int mcba_gradient(mcba_handle* h, double* d_grad) {
   return MCBA_OK;
 }
 
+int mcba_covariance(mcba_handle* h, const double* d_x, int loss, double f_scale, int ref, double sigma2,
+                    double* h_cam_cov, double* d_pose_cov, double* h_stats) {
+  int rc = need_obs(h);
+  if (rc) return rc;
+  const Layout& L = h->L;
+  if (!d_x || !h_cam_cov) { set_error("mcba_covariance: null argument"); return MCBA_ERR_ARG; }
+  if (loss != MCBA_LOSS_LINEAR && loss != MCBA_LOSS_SOFT_L1) { set_error("mcba_covariance: loss must be linear or soft_l1"); return MCBA_ERR_ARG; }
+  if (!(f_scale > 0.0)) { set_error("mcba_covariance: f_scale must be positive"); return MCBA_ERR_ARG; }
+  if (ref < 0 || ref >= L.C) {
+    set_error("mcba_covariance: reference_camera " + std::to_string(ref) + " is not in [0, " + std::to_string(L.C) + ")");
+    return MCBA_ERR_ARG;
+  }
+  if (h->nranks > 1) { set_error("mcba_covariance: frame-sharded handles are not supported"); return MCBA_ERR_STATE; }
+  int units[32];
+  MCBA_CUDA(cudaMemcpyAsync(units, h->d_unit_count, sizeof(int) * L.C, cudaMemcpyDeviceToHost, h->stream));
+  MCBA_CUDA(cudaStreamSynchronize(h->stream));
+  int observed[32], n_cam = 0;
+  for (int c = 0; c < L.C; ++c) { observed[c] = units[c] > 0; n_cam += observed[c]; }
+  if (!observed[ref]) {
+    set_error("mcba_covariance: reference camera " + std::to_string(ref) + " has no observations");
+    return MCBA_ERR_ARG;
+  }
+  EventPair e01, e23;
+  MCBA_CUDA(cudaEventCreate(&e01.a)); MCBA_CUDA(cudaEventCreate(&e01.b));
+  MCBA_CUDA(cudaEventCreate(&e23.a)); MCBA_CUDA(cudaEventCreate(&e23.b));
+  // work block: [D2pose saved | Sigma (nc^2) | Sigma_raw (nc^2) | frame check (3 x u64)]
+  const size_t n_d2 = (size_t)L.nTiles * 6 * kTile, n_cc = (size_t)L.nc * L.nc;
+  AsyncBlock blk(h->stream);
+  MCBA_CUDA(cudaMallocAsync((void**)&blk.p, sizeof(double) * (n_d2 + 2 * n_cc + 3), h->stream));
+  double* d2_saved = reinterpret_cast<double*>(blk.p);
+  double* d_cov = d2_saved + n_d2;
+  double* d_sraw = d_cov + n_cc;
+  unsigned long long* d_chk = reinterpret_cast<unsigned long long*>(d_sraw + n_cc);
+  MCBA_CUDA(cudaEventRecord(e01.a, h->stream));
+  // the evaluation starts from D2 = 0, so that D2pose afterwards holds diag V_f (the pivot test's reference);
+  // the caller's running Marquardt scaling is put back behind the check
+  MCBA_CUDA(cudaMemcpyAsync(d2_saved, h->d_D2pose, sizeof(double) * n_d2, cudaMemcpyDeviceToDevice, h->stream));
+  MCBA_CUDA(cudaMemsetAsync(h->d_D2pose, 0, sizeof(double) * n_d2, h->stream));
+  rc = evaluate(h, d_x, 0.0, loss, f_scale);
+  if (!rc) rc = launch_cov_frame_check(h, d_chk);
+  MCBA_CUDA(cudaMemcpyAsync(h->d_D2pose, d2_saved, sizeof(double) * n_d2, cudaMemcpyDeviceToDevice, h->stream));
+  if (rc) return rc;
+  MCBA_CUDA(cudaEventRecord(e01.b, h->stream));
+  double scal[kRsNum];
+  unsigned long long chk[3];
+  MCBA_CUDA(cudaMemcpyAsync(scal, h->d_red + L.offScal, sizeof(scal), cudaMemcpyDeviceToHost, h->stream));
+  MCBA_CUDA(cudaMemcpyAsync(chk, d_chk, sizeof(chk), cudaMemcpyDeviceToHost, h->stream));
+  MCBA_CUDA(cudaStreamSynchronize(h->stream));
+  const double cost = scal[kRsCost], m = scal[kRsCount];
+  double min_pivot;
+  std::memcpy(&min_pivot, &chk[2], sizeof(double));
+  auto g3 = [](double v) { char b[32]; std::snprintf(b, sizeof(b), "%.3g", v); return std::string(b); };
+  if (!std::isfinite(cost)) { set_error("Residuals are not finite at the given parameters."); return MCBA_ERR_NONFINITE; }
+  if (chk[1] > 0) {
+    set_error(std::to_string(chk[1]) + " frame(s) have a singular pose block (relative Cholesky pivot <= 1e-12, smallest " +
+              g3(min_pivot) + "): too few or collinear observed corners");
+    return MCBA_ERR_SOLVER;
+  }
+  const double p = 12.0 * n_cam + 6.0 * ((double)L.F - (double)chk[0]) - 6.0, dof = m - p;
+  double s2 = sigma2;
+  if (!(sigma2 > 0.0)) {
+    if (!(dof > 0.0)) {
+      set_error("mcba_covariance: " + std::to_string((long long)m) + " residuals do not exceed the " +
+                std::to_string((long long)p) + " free parameters; give sigma2 to use a known noise level");
+      return MCBA_ERR_ARG;
+    }
+    s2 = 2.0 * cost / dof;
+  }
+  double cam_pivot = 0.0;
+  int info = 0;
+  if ((rc = covariance_cameras(h, ref, observed, d_cov, d_sraw, &cam_pivot, &info))) return rc;
+  if (info != 0 || !(cam_pivot > kCovPivotTol)) {
+    set_error("the gauge-fixed camera system is not positive definite after Jacobi scaling (smallest relative pivot " +
+              g3(cam_pivot) + ", potrf/potri info " + std::to_string(info) + ")");
+    return MCBA_ERR_SOLVER;
+  }
+  MCBA_CUDA(cudaEventRecord(e23.a, h->stream));
+  if (d_pose_cov && (rc = launch_cov_poses(h, d_sraw, s2, d_pose_cov))) return rc;
+  MCBA_CUDA(cudaEventRecord(e23.b, h->stream));
+  MCBA_CUDA(cudaMemcpyAsync(h_cam_cov, d_cov, sizeof(double) * n_cc, cudaMemcpyDeviceToHost, h->stream));
+  MCBA_CUDA(cudaStreamSynchronize(h->stream));
+  for (size_t i = 0; i < n_cc; ++i) h_cam_cov[i] *= s2;
+  if (h_stats) {
+    float ms[3] = {0, 0, 0};
+    MCBA_CUDA(cudaEventElapsedTime(&ms[0], e01.a, e01.b));
+    MCBA_CUDA(cudaEventElapsedTime(&ms[1], e01.b, e23.a));
+    MCBA_CUDA(cudaEventElapsedTime(&ms[2], e23.a, e23.b));
+    const double st[9] = {s2, dof, m, cost, (double)chk[0], min_pivot, ms[0], ms[1], ms[2]};
+    std::memcpy(h_stats, st, sizeof(st));
+  }
+  return MCBA_OK;
+}
+
 int mcba_lm_run(mcba_handle* h, double* d_x, const mcba_options* opt_in, mcba_result* res, double* d_grad) {
   int rc = need_obs(h);
   if (rc) return rc;

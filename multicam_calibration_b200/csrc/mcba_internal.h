@@ -195,5 +195,19 @@ int launch_finalize(mcba_handle* h, bool exchange);   // exchange: sum over rank
 int launch_jacobian_blocks(mcba_handle* h, const double* x, double* Jc, double* Jp);
 int launch_backsub(mcba_handle* h, const double* x, double* x_new, double lambda);
 int allreduce_packed(mcba_handle* h, double* buf, long long n);
+int ensure_solver(mcba_handle* h);   // k3_solve.cu
+
+// calibration covariance (k8_covariance.cu, driven by mcba_covariance)
+constexpr double kCovPivotTol = 1e-12;   // relative Cholesky pivot s_j / A_jj at or below which a block is singular
+// per frame, from the factor K2c left at lambda = 0 (D2pose holding diag V_f): out[0] frames without observations,
+// out[1] observed frames with a relative pivot <= kCovPivotTol (u64), out[2] min relative pivot of the observed frames
+int launch_cov_frame_check(mcba_handle* h, unsigned long long* d_out);
+// gauge-fixed inverse of the reduced camera system in d_red: d_cov (12C x 12C, true basis, unscaled by s^2; 0 on the
+// reference camera's extrinsic rows / columns, NaN on unobserved cameras) and d_sraw = T d_cov T^T (raw basis, 0 for
+// unobserved cameras); *min_pivot = smallest relative pivot of the Jacobi-scaled Cholesky, *info = potrf's
+int covariance_cameras(mcba_handle* h, int reference_camera, const int* observed, double* d_cov, double* d_sraw,
+                       double* min_pivot, int* info);
+// per frame: s2 L^-T (I + Z^T Sigma_raw Z) L^-1 into d_pose_cov (F,6,6), caller's frame order; NaN for empty frames
+int launch_cov_poses(mcba_handle* h, const double* d_sraw, double s2, double* d_pose_cov);
 
 }  // namespace mcba

@@ -340,6 +340,42 @@ class BAProblem:
         return S, b, g, cost.value
 
     @_on_stream
+    def covariance(self, params, reference_camera=0, loss="soft_l1", f_scale=1.0, sigma=None, poses=True):
+        """Covariance of the calibration at ``params`` (``mcba_covariance``): ``(Sigma_cam (12C,12C),
+        Sigma_pose (F,6,6) or None, stats)``.
+
+        ``s^2 inv(J~^T J~)`` with J~ the residual Jacobian scaled as scipy's ``least_squares`` scales it
+        for the robust loss (``result.jac``), the extrinsics of ``reference_camera`` held fixed (exact
+        zeros), NaN for cameras and frames without observations.  ``s^2 = sigma^2``, or
+        ``2 cost / (m - p)`` with ``p`` the free parameters.  For ``loss='linear'`` this is the asymptotic
+        covariance of the least-squares estimate; for ``soft_l1`` it is scipy's usual recipe with the
+        robust-scaled Jacobian, not an M-estimator sandwich.  Singular systems raise
+        ``numpy.linalg.LinAlgError``."""
+        if loss not in ("linear", "soft_l1"):
+            raise ValueError("covariance: loss must be 'linear' or 'soft_l1'")
+        x = self._x(params)
+        nc = 12 * self.C
+        cam = np.empty((nc, nc))
+        pose = self._empty(self.F, 6, 6) if poses else None
+        stats = np.zeros(9)
+        sigma2 = -1.0 if sigma is None else float(sigma) ** 2
+        code = self.lib.mcba_covariance(
+            self._h, _ptr(x), _native.LOSSES[loss], float(f_scale), int(reference_camera), sigma2,
+            cam.ctypes.data_as(ctypes.c_void_p), _ptr(pose) if poses else None, stats.ctypes.data_as(ctypes.c_void_p))
+        if code == _native.ERR_SOLVER:
+            raise np.linalg.LinAlgError(self.lib.mcba_last_error().decode(errors="replace"))
+        if code == _native.ERR_ARG:
+            raise ValueError(self.lib.mcba_last_error().decode(errors="replace"))
+        check(code)
+        self._x_last = x
+        keys = ("sigma2", "dof", "n_residuals", "cost", "empty_frames", "min_pose_pivot",
+                "eval_ms", "camera_ms", "pose_ms")
+        info = dict(zip(keys, (float(v) for v in stats)))
+        info["n_residuals"] = int(info["n_residuals"])
+        info["empty_frames"] = int(info["empty_frames"])
+        return cam, (_native.to_host(pose) if poses else None), info
+
+    @_on_stream
     def gradient(self):
         g = self._empty(self.n_params)
         check(self.lib.mcba_gradient(self._h, _ptr(g)))
