@@ -138,6 +138,16 @@ int mcba_build_reduced_host(mcba_handle* h, const double* h_uvs, const double* h
  * Cholesky of S + lambda*D_c^2, back-substitution of every pose. d_dx: 12C + 6F. */
 int mcba_solve_step(mcba_handle* h, const double* d_x, double lambda, double* d_x_new);
 
+/* Camera parameters held at their initial values.  h_fixed: 12C bytes (host), camera-major in the order of
+ * serialize_params (fx fy cx cy k1 k2 rvec tvec), 1 = held, 0 = free; NULL or all zero = none (the solve then
+ * takes exactly the unmasked path).  Board poses are always free.  Handle state read by mcba_lm_run,
+ * mcba_solve_step and mcba_covariance until the next call.  A masked step is Levenberg-Marquardt on the free
+ * sub-problem: held rows / columns of S + lambda D^2 become the identity and their right-hand side 0, held
+ * entries of delta_cam are exactly 0 and d_x_new copies d_x there; mcba_lm_run leaves held entries out of the
+ * gtol norm, of |x| in the xtol test and of the default budget 100 n.  The gradient it returns stays complete.
+ * MCBA_ERR_ARG for an entry other than 0 / 1. */
+int mcba_set_fixed(mcba_handle* h, const uint8_t* h_fixed);
+
 /* The whole Levenberg-Marquardt loop on the device (replaces the
  * least_squares call of bundle_adjustment.py:307-313).  d_x: in x0, out solution.
  * d_grad (12C + 6F, may be NULL) receives the gradient at the solution. */
@@ -149,12 +159,17 @@ int mcba_lm_run(mcba_handle* h, double* d_x, const mcba_options* opt, mcba_resul
  * soft_l1, whatever a solve's hessian option was; lambda = 0), times the residual variance s^2.  The 6 extrinsic
  * parameters of reference_camera are held fixed (the gauge).  One evaluation (K2p, K2c, SYRK, finalize), the
  * gauge-fixed inverse of the reduced camera system and one pass over the frames.
- *   h_cam_cov   (12C x 12C, host, row major, caller's parameter basis): s^2 S^-1; exactly 0 on the reference
- *               camera's extrinsic rows / columns, NaN on the rows / columns of cameras without observations.
+ * With a mask (mcba_set_fixed) the held set is the mask together with the gauge: when the mask holds all six
+ * extrinsics of some camera no gauge is added and reference_camera must be -1 or such a camera; otherwise
+ * reference_camera is the gauge and the mask may hold no extrinsic entry (a partial extrinsic mask would leave a
+ * sub-gauge that the reference camera over-constrains).  The result is conditional on the held parameters.
+ *   h_cam_cov   (12C x 12C, host, row major, caller's parameter basis): s^2 S^-1; exactly 0 on the rows / columns
+ *               of held parameters (which wins over NaN) and of the gauge, NaN on the rows / columns of cameras
+ *               without observations.
  *   d_pose_cov  (F, 6, 6, device, may be NULL): s^2 (V^-1 + V^-1 W^T S^-1 W V^-1) per frame, [rvec | tvec];
  *               NaN for frames without observations.
  *   sigma2      > 0: s^2 = sigma2; <= 0: s^2 = 2 cost / (m - p), m finite scalar residuals,
- *               p = 12 (observed cameras) + 6 (observed frames) - 6.
+ *               p = free non-gauge parameters of the observed cameras + 6 (observed frames).
  *   h_stats     (host, may be NULL) [9]: s^2, m - p, m, cost, frames without observations, smallest relative
  *               Cholesky pivot of the observed frames' pose blocks, then device ms of {evaluation + frame check,
  *               camera inverse, pose pass}.

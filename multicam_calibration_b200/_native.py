@@ -72,6 +72,7 @@ _SIGNATURES = {
     "mcba_build_reduced": (_I, [_P, _P, _D, _I, _D, _P, _P, _P, _P]),
     "mcba_build_reduced_host": (_I, [_P, _P, _P, _P, _D, _I, _D, _P, _P, _P]),
     "mcba_solve_step": (_I, [_P, _P, _D, _P]),
+    "mcba_set_fixed": (_I, [_P, _P]),
     "mcba_gradient": (_I, [_P, _P]),
     "mcba_covariance": (_I, [_P, _P, _I, _D, _I, _D, _P, _P, _P]),
     "mcba_lm_run": (_I, [_P, _P, ctypes.POINTER(Options), ctypes.POINTER(Result), _P]),

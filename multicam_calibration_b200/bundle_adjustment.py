@@ -269,14 +269,20 @@ def bundle_adjust(all_calib_uvs, all_extrinsics, all_intrinsics, calib_objpoints
     use_frames, result)`` exactly like the reference; ``result`` has the fields of
     ``scipy.optimize.OptimizeResult`` (``jac`` is None: the Jacobian is never
     materialised).  ``opt_kwargs`` accepts ``ftol, xtol, gtol, max_nfev, loss
-    ('soft_l1' | 'linear'), f_scale, verbose``; when ``torch.distributed`` is
-    initialised with more than one rank the frames are sharded across ranks.
+    ('soft_l1' | 'linear'), f_scale, verbose``, and the engine-only ``hessian`` and
+    ``fixed``: a (C, 12) bool mask in ``serialize_params`` order of camera parameters
+    held at their initial values (e.g. ``fixed[:, :6] = True`` keeps the intrinsics,
+    ``fixed[0, 6:] = True`` keeps camera 0 where it is and so pins the gauge, all True
+    refines the board poses only); when ``torch.distributed`` is initialised with more
+    than one rank the frames are sharded across ranks.
     """
     from . import distributed
+    from .engine import check_fixed
     all_calib_uvs = np.asarray(all_calib_uvs, dtype=np.float64)
     calib_poses = np.asarray(calib_poses, dtype=np.float64)
     calib_objpoints = np.asarray(calib_objpoints, dtype=np.float64)
     n_cameras = all_calib_uvs.shape[0]
+    check_fixed(opt_kwargs.get("fixed"), n_cameras)
     if distributed.world_size() > 1:
         # every rank uploads, scans and solves only its own frames; use_frames is rank-contiguous
         use_frames, d_local, counts = _select_frames_sharded(all_calib_uvs, all_extrinsics, all_intrinsics, calib_objpoints,

@@ -34,7 +34,7 @@ def _std(diag):
 
 
 def calibration_covariance(all_calib_uvs, all_extrinsics, all_intrinsics, calib_objpoints, calib_poses,
-                           reference_camera=0, loss="soft_l1", f_scale=1.0, sigma=None, poses=True):
+                           reference_camera=0, loss="soft_l1", f_scale=1.0, sigma=None, poses=True, fixed=None):
     """Covariance of the calibration ``(all_extrinsics, all_intrinsics, calib_poses)``.
 
     The arguments are ordered like ``bundle_adjust``'s and take its outputs directly:
@@ -46,7 +46,13 @@ def calibration_covariance(all_calib_uvs, all_extrinsics, all_intrinsics, calib_
     other parameter in that camera's frame, and the reference camera's extrinsic rows and columns are 0.
     Cameras and frames without any finite observation are NaN.  The residual variance is ``sigma**2`` when
     ``sigma`` (px) is given, else ``2 cost / (m - p)``: m finite residual scalars, p = 12 observed cameras
-    + 6 observed frames - 6.
+    + 6 observed frames - 6 (with a mask: the free non-gauge parameters of the observed cameras + 6 observed frames).
+
+    ``fixed`` (C, 12) bool, ``serialize_params`` order: parameters held fixed in the solve (``bundle_adjust``'s
+    ``fixed``).  The result is conditional on them: their rows and columns are exactly 0, also for a camera
+    without observations, and p counts the free parameters only.  A mask that holds all six extrinsics of some
+    camera fixes the gauge itself: ``reference_camera`` must then be None or such a camera.  Otherwise the
+    reference camera is the gauge, and the mask may hold no extrinsic entry.
 
     For ``loss='linear'`` this is the asymptotic covariance of the least-squares estimate.  For ``soft_l1``
     it is scipy's usual recipe applied to the robust-scaled Jacobian, not an M-estimator sandwich
@@ -58,15 +64,19 @@ def calibration_covariance(all_calib_uvs, all_extrinsics, all_intrinsics, calib_
     ``torch.distributed`` is initialised.
     """
     from .bundle_adjustment import _problem_for, serialize_params
+    from .engine import check_fixed
 
     uvs = all_calib_uvs if hasattr(all_calib_uvs, "is_cuda") else np.asarray(all_calib_uvs, dtype=np.float64)
     if uvs.ndim != 4 or uvs.shape[-1] != 2:
         raise ValueError("all_calib_uvs must be (C, F, N, 2)")
     C, F = int(uvs.shape[0]), int(uvs.shape[1])
-    if isinstance(reference_camera, (bool, np.bool_)) or not isinstance(reference_camera, (int, np.integer)):
-        raise ValueError("reference_camera must be an integer camera index")
-    if not 0 <= int(reference_camera) < C:
-        raise ValueError(f"reference_camera {reference_camera} is not in [0, {C})")
+    if reference_camera is not None:
+        if isinstance(reference_camera, (bool, np.bool_)) or not isinstance(reference_camera, (int, np.integer)):
+            raise ValueError("reference_camera must be None or an integer camera index")
+        if not 0 <= int(reference_camera) < C:
+            raise ValueError(f"reference_camera {reference_camera} is not in [0, {C})")
+        reference_camera = int(reference_camera)
+    check_fixed(fixed, C)
     if loss not in ("linear", "soft_l1"):
         raise ValueError("loss must be 'linear' or 'soft_l1'")
     if not (np.isfinite(f_scale) and f_scale > 0):
@@ -83,8 +93,8 @@ def calibration_covariance(all_calib_uvs, all_extrinsics, all_intrinsics, calib_
         raise ValueError("Residuals are not finite at the given parameters (non-finite parameters).")
 
     prob = _problem_for(uvs, calib_objpoints)
-    cam, pose, info = prob.covariance(x, reference_camera=int(reference_camera), loss=loss, f_scale=float(f_scale),
-                                      sigma=sigma, poses=poses)
+    cam, pose, info = prob.covariance(x, reference_camera=reference_camera, loss=loss, f_scale=float(f_scale),
+                                      sigma=sigma, poses=poses, fixed=fixed)
     return CalibrationCovariance(
         camera=cam, camera_std=_std(np.diag(cam)).reshape(C, 12),
         poses=pose, pose_std=None if pose is None else _std(np.einsum("fii->fi", pose)),

@@ -710,6 +710,7 @@ struct BackParams {
   const double* Z; const double* Linv; const double* y; const double* gpose; const double* D2pose;
   const double* D2cam; const double* gcam;
   double* part; unsigned int* counter; double* out;  // out[0..3] = |dx|^2, |x|^2, g.dx, dx D2 dx
+  const uint8_t* fixed; // [nc] held camera parameters: x copied, left out of the scalars (nullptr = none)
 };
 
 __global__ void __launch_bounds__(kBackWarps * 32, 1) backsub_kernel(const BackParams p) {
@@ -827,6 +828,7 @@ __global__ void __launch_bounds__(kBackWarps * 32, 1) backsub_kernel(const BackP
   if (blockIdx.x == 0 && warp == 0) {
     for (int r = lane; r < nc; r += 32) {
       const double d = p.dcam[r], xo = p.x[r];
+      if (p.fixed && p.fixed[r]) { p.x_new[r] = xo; continue; }   // a copy: -0.0 survives
       p.x_new[r] = xo + d;
       if (p.rank == 0) {  // camera terms are counted once across ranks
         double d2 = p.D2cam[r];
@@ -889,6 +891,7 @@ int launch_backsub(mcba_handle* h, const double* x, double* x_new, double lambda
   p.cams = h->d_cams; p.perm = h->d_perm; p.active = h->d_active; p.x = x; p.x_new = x_new; p.dcam = h->d_dcam;
   p.Z = h->d_Z; p.Linv = h->d_Linv; p.y = h->d_y; p.gpose = h->d_gpose; p.D2pose = h->d_D2pose;
   p.D2cam = h->d_D2cam; p.gcam = h->d_red + L.offG;
+  p.fixed = h->any_fixed ? h->d_fixed : nullptr;
   p.part = h->d_scal + 64 + 3 * 4096;                                     // [grid_back][4]
   p.counter = reinterpret_cast<unsigned int*>(h->d_scal + 33);
   p.out = h->d_scal + 8;

@@ -68,6 +68,7 @@ struct SolveParams {
   double* D2cam;        // running max of diag(U) (Marquardt scaling), updated here
   double* dcam;         // out: delta_cam (true basis), nc
   int* info;            // out: 0, or 1 + index of the first non-positive pivot
+  const uint8_t* fixed; // [nc] held parameters (mcba_set_fixed): identity row / column, 0 right-hand side; nullptr = none
 };
 
 // kT: trailing tiles per warp (3: up to 6 cameras, 8: up to 10, 19: up to 16 -- 24 * 25 / 2 = 300 tiles of the
@@ -109,8 +110,9 @@ __global__ void __launch_bounds__(kSolveThreads, 1) solve_reduced_kernel(const S
         const int pr = e / pw, off = e - pr * pw;
         const int i = off <= pr ? pr : n1p - 1 - pr, j = off <= pr ? off : off - pr - 1;
         at[u] = pk(i, j);
-        if (i < nc) v[u] = __ldcg(p.red + p.offS + (size_t)i * nc + j);
-        else if (i == nc) v[u] = j < nc ? -__ldcg(p.red + p.offB + j) : 1.0;
+        const bool held_j = p.fixed && j < nc && p.fixed[j];
+        if (i < nc) v[u] = held_j || (p.fixed && p.fixed[i]) ? (i == j ? 1.0 : 0.0) : __ldcg(p.red + p.offS + (size_t)i * nc + j);
+        else if (i == nc) v[u] = j < nc ? (held_j ? 0.0 : -__ldcg(p.red + p.offB + j)) : 1.0;
         else v[u] = i == j ? 1.0 : 0.0;
       }
     }
@@ -269,7 +271,7 @@ __global__ void __launch_bounds__(kSolveThreads, 1) solve_reduced_kernel(const S
     }
 #pragma unroll
     for (int s = 0; s < kSlots; ++s)
-      if (lane + 32 * s < nc) p.dcam[lane + 32 * s] = y[s];
+      if (lane + 32 * s < nc) p.dcam[lane + 32 * s] = p.fixed && p.fixed[lane + 32 * s] ? 0.0 : y[s];
     if (lane == 0) p.info[0] = s_info;
     MCBA_STAMP(4);
   }
@@ -278,17 +280,18 @@ __global__ void __launch_bounds__(kSolveThreads, 1) solve_reduced_kernel(const S
 // ------------------------------------------------------------------ library path (12C > 192, or MCBA_CUSOLVER=1 for A/B runs)
 __global__ void damp_kernel(const double* __restrict__ red, long long offS, long long offB, long long offDiag,
                             int nc, double lambda, double* __restrict__ D2cam, double* __restrict__ Sd,
-                            double* __restrict__ rhs) {
+                            double* __restrict__ rhs, const uint8_t* __restrict__ fixed) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= nc * nc) return;
   const int r = i / nc, q = i % nc;
-  double v = red[offS + i];
+  const bool held = fixed && (fixed[r] || fixed[q]);   // identity row / column, 0 right-hand side: delta = 0 there
+  double v = held ? 0.0 : red[offS + i];
   if (r == q) {
     double d2 = fmax(D2cam[r], red[offDiag + r]);
     D2cam[r] = d2;
     if (d2 == 0.0) d2 = 1.0;
-    v = fma(lambda, d2, v);
-    rhs[r] = -red[offB + r];
+    v = held ? 1.0 : fma(lambda, d2, v);
+    rhs[r] = held ? 0.0 : -red[offB + r];
   }
   Sd[i] = v;
 }
@@ -332,7 +335,7 @@ int solve_reduced(mcba_handle* h, double lambda) {
   if (tier != kSolveTierLibrary) {
     SolveParams p;
     p.red = h->d_red; p.offS = L.offS; p.offB = L.offB; p.offDiag = L.offDiag; p.nc = nc; p.lambda = lambda;
-    p.D2cam = h->d_D2cam; p.dcam = h->d_dcam; p.info = h->d_info;
+    p.D2cam = h->d_D2cam; p.dcam = h->d_dcam; p.info = h->d_info; p.fixed = h->any_fixed ? h->d_fixed : nullptr;
     const int n1p = (nc + 1 + 7) & ~7;
     const size_t smem = sizeof(double) * (size_t)n1p * (n1p + 1) / 2;
 #define MCBA_SOLVE(...)                                                                                                    \
@@ -360,7 +363,7 @@ int solve_reduced(mcba_handle* h, double lambda) {
   int rc = ensure_solver(h);
   if (rc) return rc;
   damp_kernel<<<(nc * nc + 255) / 256, 256, 0, h->stream>>>(h->d_red, L.offS, L.offB, L.offDiag, nc, lambda,
-                                                            h->d_D2cam, h->d_Sd, h->d_dcam);
+                                                            h->d_D2cam, h->d_Sd, h->d_dcam, h->any_fixed ? h->d_fixed : nullptr);
   h->launches++;
   MCBA_CUDA(cudaGetLastError());
   cusolverStatus_t st = cusolverDnDpotrf(h->solver, CUBLAS_FILL_MODE_LOWER, nc, h->d_Sd, nc, h->d_work, h->lwork, h->d_info);

@@ -94,13 +94,14 @@ __global__ void cov_pivot_kernel(const double* __restrict__ A, int nk, double* _
 }
 
 // Sigma (nc x nc, true basis) from the inverse of A (lower triangle, column-major): pos[r] = row of A, -1 gauge,
-// -2 unobserved camera
+// -2 unobserved camera, -3 held parameter (0, also against an unobserved camera)
 __global__ void cov_expand_kernel(const double* __restrict__ Ainv, int nk, const double* __restrict__ rs,
                                   const int* __restrict__ pos, int nc, double* __restrict__ cov) {
   for (int e = blockIdx.x * blockDim.x + threadIdx.x; e < nc * nc; e += gridDim.x * blockDim.x) {
     const int pr = pos[e / nc], pq = pos[e % nc];
     double v;
-    if (pr == -2 || pq == -2) v = NAN;
+    if (pr == -3 || pq == -3) v = 0.0;
+    else if (pr == -2 || pq == -2) v = NAN;
     else if (pr < 0 || pq < 0) v = 0.0;
     else v = Ainv[(size_t)min(pr, pq) * nk + max(pr, pq)] * rs[pr] * rs[pq];
     cov[e] = v;
@@ -137,18 +138,34 @@ __global__ void cov_raw_kernel(const double* __restrict__ cov, const CamConst* _
   }
 }
 
-int covariance_cameras(mcba_handle* h, int ref, const int* observed, double* d_cov, double* d_sraw, double* min_pivot,
-                       int* info) {
+int covariance_cameras(mcba_handle* h, int ref, const int* observed, const uint8_t* held, double* d_cov, double* d_sraw,
+                       double* min_pivot, int* info) {
   const Layout& L = h->L;
   const int nc = L.nc;
   std::vector<int> keep, pos(nc);
   for (int r = 0; r < nc; ++r) {
     const int c = r / 12;
-    if (!observed[c]) pos[r] = -2;
+    if (held && held[r]) pos[r] = -3;
+    else if (!observed[c]) pos[r] = -2;
     else if (c == ref && r % 12 >= 6) pos[r] = -1;
     else { pos[r] = (int)keep.size(); keep.push_back(r); }
   }
   const int nk = (int)keep.size();
+  const int grid = (nc * nc + 255) / 256;
+  if (nk == 0) {   // every camera parameter held: nothing to invert, Sigma is 0 / NaN and Sigma_raw 0
+    AsyncBlock blk(h->stream);
+    MCBA_CUDA(cudaMallocAsync((void**)&blk.p, sizeof(int) * nc, h->stream));
+    int* d_pos = reinterpret_cast<int*>(blk.p);
+    MCBA_CUDA(cudaMemcpyAsync(d_pos, pos.data(), sizeof(int) * nc, cudaMemcpyHostToDevice, h->stream));
+    cov_expand_kernel<<<grid, 256, 0, h->stream>>>(nullptr, 0, nullptr, d_pos, nc, d_cov);
+    cov_raw_kernel<<<grid, 256, 0, h->stream>>>(d_cov, h->d_cams, nc, d_sraw);
+    h->launches += 2;
+    MCBA_CUDA(cudaGetLastError());
+    MCBA_CUDA(cudaStreamSynchronize(h->stream));   // pos is a host vector
+    *min_pivot = INFINITY;
+    *info = 0;
+    return MCBA_OK;
+  }
   int rc = ensure_solver(h);
   if (rc) return rc;
   int lw_f = 0, lw_i = 0;
@@ -185,7 +202,6 @@ int covariance_cameras(mcba_handle* h, int ref, const int* observed, double* d_c
     set_error("cusolverDnDpotri failed");
     return MCBA_ERR_SOLVER;
   }
-  const int grid = (nc * nc + 255) / 256;
   cov_expand_kernel<<<grid, 256, 0, h->stream>>>(A, nk, rs, d_pos, nc, d_cov);
   cov_raw_kernel<<<grid, 256, 0, h->stream>>>(d_cov, h->d_cams, nc, d_sraw);
   h->launches += 6;   // compact, potrf, pivot, potri, expand, raw (library calls counted once)

@@ -270,7 +270,8 @@ static void parse_eval(mcba_handle* h, EvalOut* out) {
   const double* sc = t + (L.offScal - L.offB);
   const double* rk = t + (L.offRank - L.offB);
   double gn = 0.0;
-  for (int i = 0; i < L.nc; ++i) gn = std::max(gn, std::fabs(g[i]));
+  for (int i = 0; i < L.nc; ++i)   // gtol / optimality of the free sub-problem: held entries do not count
+    if (!h->any_fixed || !h->h_fixed[i]) gn = std::max(gn, std::fabs(g[i]));
   bool bad = false;
   for (int i = 0; i < L.nc; ++i) bad |= !std::isfinite(g[i]);
   for (int i = 0; i < kMaxRanks; ++i) gn = std::max(gn, rk[i]);
@@ -432,7 +433,7 @@ int mcba_destroy(mcba_handle* h) {
   if (h->peer_block) cudaFree(h->peer_block);
   void* ptrs[] = {h->d_obs_ref, h->d_obs_tiled, h->d_obj, h->d_row_off, h->d_x, h->d_xtrial, h->d_cams, h->d_Z,
                   h->d_Linv, h->d_y, h->d_JlTau, h->d_gpose, h->d_D2pose, h->d_D2cam, h->d_partU, h->d_partS, h->d_partSyrk,
-                  h->d_red, h->d_Sd, h->d_dcam, h->d_scal, h->d_info, h->d_work, h->d_Sraw, h->d_H, h->d_H_alt, h->d_partU_alt, h->d_partS_alt, h->d_cams_alt, h->d_partG, h->d_partZy, h->d_perm, h->d_mask, h->d_active, h->d_sort_tmp, h->d_units, h->d_unit_count, h->d_rowT, h->d_chunk_rows, h->d_fin_scratch, h->d_fin_counter};
+                  h->d_red, h->d_Sd, h->d_dcam, h->d_scal, h->d_info, h->d_work, h->d_Sraw, h->d_H, h->d_H_alt, h->d_partU_alt, h->d_partS_alt, h->d_cams_alt, h->d_partG, h->d_partZy, h->d_perm, h->d_mask, h->d_active, h->d_sort_tmp, h->d_units, h->d_unit_count, h->d_rowT, h->d_chunk_rows, h->d_fin_scratch, h->d_fin_counter, h->d_fixed};
   for (void* p : ptrs) if (p) cudaFree(p);
   if (h->prof_ev) {
     for (int i = 0; i < kProfEvents * kProfRing; ++i) cudaEventDestroy(h->prof_ev[i]);
@@ -854,6 +855,31 @@ int mcba_gradient(mcba_handle* h, double* d_grad) {
   return MCBA_OK;
 }
 
+int mcba_set_fixed(mcba_handle* h, const uint8_t* h_fixed) {
+  if (!h) return MCBA_ERR_ARG;
+  MCBA_CUDA(cudaSetDevice(h->device));
+  const int nc = h->L.nc;
+  bool any = false;
+  if (h_fixed) {
+    for (int i = 0; i < nc; ++i) {
+      if (h_fixed[i] > 1) {
+        set_error("mcba_set_fixed: entry " + std::to_string(i) + " is " + std::to_string((int)h_fixed[i]) +
+                  "; entries must be 0 (free) or 1 (held)");
+        return MCBA_ERR_ARG;
+      }
+      any |= h_fixed[i] != 0;
+    }
+  }
+  // the kernels of work already queued may still read the previous mask
+  MCBA_CUDA(cudaStreamSynchronize(h->stream));
+  h->any_fixed = any;
+  if (!any) { std::memset(h->h_fixed, 0, sizeof(h->h_fixed)); return MCBA_OK; }
+  std::memcpy(h->h_fixed, h_fixed, nc);
+  if (!h->d_fixed) MCBA_CUDA(cudaMalloc((void**)&h->d_fixed, nc));
+  MCBA_CUDA(cudaMemcpyAsync(h->d_fixed, h->h_fixed, nc, cudaMemcpyHostToDevice, h->stream));
+  return MCBA_OK;
+}
+
 int mcba_covariance(mcba_handle* h, const double* d_x, int loss, double f_scale, int ref, double sigma2,
                     double* h_cam_cov, double* d_pose_cov, double* h_stats) {
   int rc = need_obs(h);
@@ -862,18 +888,46 @@ int mcba_covariance(mcba_handle* h, const double* d_x, int loss, double f_scale,
   if (!d_x || !h_cam_cov) { set_error("mcba_covariance: null argument"); return MCBA_ERR_ARG; }
   if (loss != MCBA_LOSS_LINEAR && loss != MCBA_LOSS_SOFT_L1) { set_error("mcba_covariance: loss must be linear or soft_l1"); return MCBA_ERR_ARG; }
   if (!(f_scale > 0.0)) { set_error("mcba_covariance: f_scale must be positive"); return MCBA_ERR_ARG; }
-  if (ref < 0 || ref >= L.C) {
-    set_error("mcba_covariance: reference_camera " + std::to_string(ref) + " is not in [0, " + std::to_string(L.C) + ")");
+  if (ref < -1 || ref >= L.C) {
+    set_error("mcba_covariance: reference_camera " + std::to_string(ref) + " is not -1 or in [0, " + std::to_string(L.C) + ")");
+    return MCBA_ERR_ARG;
+  }
+  // the gauge: a camera whose six extrinsics the mask holds pins it; otherwise the reference camera's extrinsics
+  const uint8_t* held = h->any_fixed ? h->h_fixed : nullptr;
+  auto pinned = [&](int c) {
+    if (!held) return false;
+    for (int k = 6; k < 12; ++k) if (!held[12 * c + k]) return false;
+    return true;
+  };
+  bool any_pinned = false, any_extrinsic = false;
+  for (int c = 0; c < L.C; ++c) {
+    any_pinned |= pinned(c);
+    for (int k = 6; k < 12; ++k) any_extrinsic |= held && held[12 * c + k];
+  }
+  int gauge = ref;
+  if (any_pinned) {
+    if (ref >= 0 && !pinned(ref)) {
+      set_error("mcba_covariance: the mask holds all six extrinsics of a camera, which fixes the gauge; reference_camera " +
+                std::to_string(ref) + " is not such a camera (give -1 / None, or a pinned camera)");
+      return MCBA_ERR_ARG;
+    }
+    gauge = -1;
+  } else if (ref < 0) {
+    set_error("mcba_covariance: reference_camera is -1 / None but no camera has all six extrinsics held: the gauge is not fixed");
+    return MCBA_ERR_ARG;
+  } else if (any_extrinsic) {
+    set_error("mcba_covariance: the mask holds some extrinsic parameters but no camera's complete set; with the reference "
+              "camera as the gauge that over-constrains the problem (hold all six extrinsics of one camera instead)");
     return MCBA_ERR_ARG;
   }
   if (h->nranks > 1) { set_error("mcba_covariance: frame-sharded handles are not supported"); return MCBA_ERR_STATE; }
   int units[32];
   MCBA_CUDA(cudaMemcpyAsync(units, h->d_unit_count, sizeof(int) * L.C, cudaMemcpyDeviceToHost, h->stream));
   MCBA_CUDA(cudaStreamSynchronize(h->stream));
-  int observed[32], n_cam = 0;
-  for (int c = 0; c < L.C; ++c) { observed[c] = units[c] > 0; n_cam += observed[c]; }
-  if (!observed[ref]) {
-    set_error("mcba_covariance: reference camera " + std::to_string(ref) + " has no observations");
+  int observed[32];
+  for (int c = 0; c < L.C; ++c) observed[c] = units[c] > 0;
+  if (gauge >= 0 && !observed[gauge]) {
+    set_error("mcba_covariance: reference camera " + std::to_string(gauge) + " has no observations");
     return MCBA_ERR_ARG;
   }
   EventPair e01, e23;
@@ -912,7 +966,10 @@ int mcba_covariance(mcba_handle* h, const double* d_x, int loss, double f_scale,
               g3(min_pivot) + "): too few or collinear observed corners");
     return MCBA_ERR_SOLVER;
   }
-  const double p = 12.0 * n_cam + 6.0 * ((double)L.F - (double)chk[0]) - 6.0, dof = m - p;
+  long long p_cam = 0;   // free non-gauge parameters of the observed cameras
+  for (int r = 0; r < L.nc; ++r)
+    p_cam += observed[r / 12] && !(held && held[r]) && !(r / 12 == gauge && r % 12 >= 6);
+  const double p = (double)p_cam + 6.0 * ((double)L.F - (double)chk[0]), dof = m - p;
   double s2 = sigma2;
   if (!(sigma2 > 0.0)) {
     if (!(dof > 0.0)) {
@@ -924,7 +981,7 @@ int mcba_covariance(mcba_handle* h, const double* d_x, int loss, double f_scale,
   }
   double cam_pivot = 0.0;
   int info = 0;
-  if ((rc = covariance_cameras(h, ref, observed, d_cov, d_sraw, &cam_pivot, &info))) return rc;
+  if ((rc = covariance_cameras(h, gauge, observed, held, d_cov, d_sraw, &cam_pivot, &info))) return rc;
   if (info != 0 || !(cam_pivot > kCovPivotTol)) {
     set_error("the gauge-fixed camera system is not positive definite after Jacobi scaling (smallest relative pivot " +
               g3(cam_pivot) + ", potrf/potri info " + std::to_string(info) + ")");
@@ -992,14 +1049,17 @@ int mcba_lm_run(mcba_handle* h, double* d_x, const mcba_options* opt_in, mcba_re
   // The TOTAL parameter count decides the default evaluation budget (scipy: 100 n).  With uneven
   // shards 6 F differs between ranks, and a rank-local budget would let one rank leave the loop --
   // and the collective -- before the others: sum the pose counts over the ranks once.
-  long long n_total = n_local;
+  // Held camera parameters are not parameters of the sub-problem (every rank holds the same mask).
+  long long n_cam_free = L.nc;
+  if (h->any_fixed) for (int i = 0; i < L.nc; ++i) n_cam_free -= h->h_fixed[i];
+  long long n_total = n_cam_free + 6 * L.F;
   if (h->nranks > 1 && opt.max_nfev <= 0) {
     const double mine = 6.0 * (double)L.F;
     MCBA_CUDA(cudaMemcpyAsync(h->d_scal + 40, &mine, sizeof(double), cudaMemcpyHostToDevice, h->stream));
     if ((rc = allreduce_packed(h, h->d_scal + 40, 1))) return rc;
     MCBA_CUDA(cudaMemcpyAsync(h->h_pinned + L.redLen, h->d_scal + 40, sizeof(double), cudaMemcpyDeviceToHost, h->stream));
     MCBA_CUDA(cudaStreamSynchronize(h->stream));
-    n_total = L.nc + (long long)h->h_pinned[L.redLen];
+    n_total = n_cam_free + (long long)h->h_pinned[L.redLen];
   }
   int max_nfev = opt.max_nfev > 0 ? opt.max_nfev : (int)std::min<long long>(100 * n_total, 2000000000LL);
   double cost = ev.cost;

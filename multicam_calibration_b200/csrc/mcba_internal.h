@@ -101,6 +101,11 @@ struct mcba_handle {
   double* d_Sd = nullptr;     // damped copy handed to potrf
   double* d_dcam = nullptr;   // [delta_cam true (12C) | delta_cam raw (12C)]
   double* d_scal = nullptr;   // step scalars (device), partials
+  // camera parameters held at their initial values (mcba_set_fixed): 12C bytes, 0 / 1; the kernels get
+  // d_fixed only while some entry is held (nullptr: the unmasked path)
+  uint8_t h_fixed[12 * 32] = {};
+  uint8_t* d_fixed = nullptr;
+  bool any_fixed = false;
   double* h_pinned = nullptr; // pinned host mirror for small read-backs
   // mapped pinned block the LM loop polls: [16 doubles | sequence flag]; device aliases of the same memory
   double* h_signal_vals = nullptr;
@@ -203,10 +208,12 @@ constexpr double kCovPivotTol = 1e-12;   // relative Cholesky pivot s_j / A_jj a
 // out[1] observed frames with a relative pivot <= kCovPivotTol (u64), out[2] min relative pivot of the observed frames
 int launch_cov_frame_check(mcba_handle* h, unsigned long long* d_out);
 // gauge-fixed inverse of the reduced camera system in d_red: d_cov (12C x 12C, true basis, unscaled by s^2; 0 on the
-// reference camera's extrinsic rows / columns, NaN on unobserved cameras) and d_sraw = T d_cov T^T (raw basis, 0 for
-// unobserved cameras); *min_pivot = smallest relative pivot of the Jacobi-scaled Cholesky, *info = potrf's
-int covariance_cameras(mcba_handle* h, int reference_camera, const int* observed, double* d_cov, double* d_sraw,
-                       double* min_pivot, int* info);
+// rows / columns of held parameters (held[r], may be null; wins over NaN) and of the reference camera's extrinsics
+// (none for reference_camera = -1), NaN on unobserved cameras) and d_sraw = T d_cov T^T (raw basis, 0 for unobserved
+// cameras); *min_pivot = smallest relative pivot of the Jacobi-scaled Cholesky (+inf when nothing is left to
+// invert), *info = potrf's
+int covariance_cameras(mcba_handle* h, int reference_camera, const int* observed, const uint8_t* held, double* d_cov,
+                       double* d_sraw, double* min_pivot, int* info);
 // per frame: s2 L^-T (I + Z^T Sigma_raw Z) L^-1 into d_pose_cov (F,6,6), caller's frame order; NaN for empty frames
 int launch_cov_poses(mcba_handle* h, const double* d_sraw, double s2, double* d_pose_cov);
 

@@ -100,6 +100,22 @@ def _on_stream(fn):
     return wrapper
 
 
+def check_fixed(fixed, n_cameras):
+    """``fixed`` (camera parameters held at their initial values, ``serialize_params`` order) as the 12C
+    bytes of ``mcba_set_fixed``, or None when nothing is held (None or an all-False mask)."""
+    if fixed is None:
+        return None
+    mask = np.asarray(fixed)
+    if mask.dtype != np.bool_:
+        raise ValueError(f"fixed must be a boolean array, got dtype {mask.dtype}")
+    if mask.shape != (n_cameras, 12):
+        raise ValueError(f"fixed must have shape ({n_cameras}, 12) (fx fy cx cy k1 k2 rvec tvec per camera), "
+                         f"got {mask.shape}")
+    if not mask.any():
+        return None
+    return np.ascontiguousarray(mask, dtype=np.uint8).ravel()
+
+
 def parse_options(opt_kwargs, n_params):
     """Map ``least_squares`` keyword arguments (bundle_adjustment.py:301-304) to
     :class:`Options`; scipy-only knobs the engine replaces are rejected loudly."""
@@ -340,7 +356,15 @@ class BAProblem:
         return S, b, g, cost.value
 
     @_on_stream
-    def covariance(self, params, reference_camera=0, loss="soft_l1", f_scale=1.0, sigma=None, poses=True):
+    def set_fixed(self, fixed):
+        """Hold camera parameters at their initial values in the following :meth:`solve_step` calls
+        (``mcba_set_fixed``): ``fixed`` (C, 12) bool in ``serialize_params`` order, or None.  :meth:`solve` and
+        :meth:`covariance` set their own mask on every call."""
+        mask = check_fixed(fixed, self.C)
+        check(self.lib.mcba_set_fixed(self._h, None if mask is None else mask.ctypes.data_as(ctypes.c_void_p)))
+
+    @_on_stream
+    def covariance(self, params, reference_camera=0, loss="soft_l1", f_scale=1.0, sigma=None, poses=True, fixed=None):
         """Covariance of the calibration at ``params`` (``mcba_covariance``): ``(Sigma_cam (12C,12C),
         Sigma_pose (F,6,6) or None, stats)``.
 
@@ -350,17 +374,22 @@ class BAProblem:
         ``2 cost / (m - p)`` with ``p`` the free parameters.  For ``loss='linear'`` this is the asymptotic
         covariance of the least-squares estimate; for ``soft_l1`` it is scipy's usual recipe with the
         robust-scaled Jacobian, not an M-estimator sandwich.  Singular systems raise
-        ``numpy.linalg.LinAlgError``."""
+        ``numpy.linalg.LinAlgError``.
+
+        ``fixed`` (C, 12) bool: parameters held fixed, conditioned on (their rows and columns are exactly 0).
+        When it holds all six extrinsics of a camera that fixes the gauge, and ``reference_camera`` must be None
+        or such a camera; otherwise the mask may hold no extrinsic entry."""
         if loss not in ("linear", "soft_l1"):
             raise ValueError("covariance: loss must be 'linear' or 'soft_l1'")
         x = self._x(params)
+        self.set_fixed(fixed)
         nc = 12 * self.C
         cam = np.empty((nc, nc))
         pose = self._empty(self.F, 6, 6) if poses else None
         stats = np.zeros(9)
         sigma2 = -1.0 if sigma is None else float(sigma) ** 2
         code = self.lib.mcba_covariance(
-            self._h, _ptr(x), _native.LOSSES[loss], float(f_scale), int(reference_camera), sigma2,
+            self._h, _ptr(x), _native.LOSSES[loss], float(f_scale), -1 if reference_camera is None else int(reference_camera), sigma2,
             cam.ctypes.data_as(ctypes.c_void_p), _ptr(pose) if poses else None, stats.ctypes.data_as(ctypes.c_void_p))
         if code == _native.ERR_SOLVER:
             raise np.linalg.LinAlgError(self.lib.mcba_last_error().decode(errors="replace"))
@@ -402,9 +431,14 @@ class BAProblem:
 
     # ------------------------------------------------------------------ the solve
     @_on_stream
-    def solve(self, x0, **opt_kwargs):
-        """Levenberg-Marquardt on the device; returns ``(x, OptimizeResult)``."""
+    def solve(self, x0, fixed=None, **opt_kwargs):
+        """Levenberg-Marquardt on the device; returns ``(x, OptimizeResult)``.
+
+        ``fixed`` (C, 12) bool, ``serialize_params`` order: camera parameters held at their values in ``x0``
+        (Levenberg-Marquardt on the free sub-problem; ``optimality`` and the default ``max_nfev`` count free
+        parameters only, ``grad`` stays complete)."""
         opts = parse_options(opt_kwargs, self.n_params)
+        self.set_fixed(fixed)
         verbose = opts.verbose if self.rank == 0 else 0
         keep = []
         if verbose >= 2:
