@@ -298,8 +298,10 @@ __global__ void __launch_bounds__(128) triangulate_kernel(const double* __restri
     bool seen[kMaxC];
     for (int c = 0; c < C; ++c) {
       const double2 o = reinterpret_cast<const double2*>(uvs)[(long long)c * P + pt];
-      seen[c] = (o.x == o.x) && (o.y == o.y);
       undistort5(sc[c], o.x, o.y, und[c][0], und[c][1]);
+      // seen from the undistorted pixel, as the reference's triangulate decides it: a NaN input stays
+      // NaN, and an infinite or overflowing one (+-inf, 1e300) undistorts to NaN and enters no pair
+      seen[c] = (und[c][0] == und[c][0]) && (und[c][1] == und[c][1]);
     }
     double px[kMaxPairs], py[kMaxPairs], pz[kMaxPairs];
     int np = 0;
