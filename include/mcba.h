@@ -280,6 +280,38 @@ int mcba_triangulate(int device, void* cuda_stream, const double* d_uvs, int n_c
                      int64_t n_points, const double* h_ext, const double* h_K,
                      const double* h_dist, double* d_points);
 
+/* Refinement of triangulated points (geometry.refine_points): per point, Levenberg-Marquardt on
+ *   0.5 sum_views sum_{u,v} f_scale^2 rho((f / f_scale)^2),  f = observed - project_points(X, ext_c, K_c, k1_c, k2_c)
+ * (fx, skew, cx, fy, cy of K; k1, k2 of dist), with scipy's robust losses and its ftol / xtol / gtol tests
+ * (least_squares.py:183-219, common.py:705-731) applied per point.  A view is seen when its pixel undistorts
+ * to a finite point with the 5-coefficient model, as mcba_triangulate decides it.  These loss codes are this
+ * call's own; the bundle-adjustment entry points keep MCBA_LOSS_*. */
+#define MCBA_REFINE_LOSS_LINEAR 0
+#define MCBA_REFINE_LOSS_SOFT_L1 1
+#define MCBA_REFINE_LOSS_HUBER 2
+#define MCBA_REFINE_LOSS_CAUCHY 3
+#define MCBA_REFINE_LOSS_ARCTAN 4
+typedef struct mcba_refine_options {
+  int32_t loss;     /* MCBA_REFINE_LOSS_* */
+  double f_scale;   /* > 0 */
+  double sigma;     /* > 0: pixel noise of the covariance, sigma^2 inv(J~^T J~) */
+  double ftol, xtol, gtol;
+  int32_t max_iter; /* 1 .. 32767 trial steps per point */
+  int32_t flags;    /* reserved, 0 */
+} mcba_refine_options;
+/* d_uvs (C,P,2) NaN = missing, h_ext (C,6), h_K (C,3,3), h_dist (C,5); d_init (P,3) start, or NULL for the
+ * mcba_triangulate result computed in the call.  Outputs (device): d_points (P,3) (may be d_init), d_cost (P)
+ * 0.5 sum rho, d_rms (P) reprojection RMS over the point's scalars, d_status (P) {1 gtol, 2 ftol, 3 xtol,
+ * 4 ftol + xtol, 0 max_iter, -1 fewer than two seen views (point NaN), -2 non-finite start or cost at the
+ * start, or damping beyond its bound (start returned)}, d_iters (P) trial steps, d_cov (P,6) upper triangle
+ * xx xy xz yy yz zz of sigma^2 inv(J~^T J~) at the result, J~ scaled as scipy's result.jac (may be NULL),
+ * d_view_err (C,P) reprojection distance per view, NaN where unseen (may be NULL), d_n_views (P) seen views
+ * (may be NULL).  1 <= C <= 32. */
+int mcba_refine_points(int device, void* cuda_stream, const double* d_uvs, int n_cameras, int64_t n_points,
+                       const double* h_ext, const double* h_K, const double* h_dist, const double* d_init,
+                       const mcba_refine_options* opt, double* d_points, double* d_cost, double* d_rms,
+                       int8_t* d_status, int16_t* d_iters, double* d_cov, double* d_view_err, int8_t* d_n_views);
+
 /* ---- reprojection-error QC (the step after bundle_adjust; viz.py:155-177 plot_residuals) ----
  * Per camera and frame whose N corners were all detected: undistort the detections (geometry.py:328-358),
  * homography detections -> board plane as cv2.findHomography computes it (float32-rounded points,

@@ -5,13 +5,15 @@
 reference builds with its star imports (``multicam_calibration/__init__.py:1-7``)
 for the two hot-path modules, plus the steps on either side of them: the rigid-transform part of
 ``calibration`` that produces bundle_adjust's initial guess (calibration.py:116-277), the
-reprojection-error check of its result (viz.py:70-210) and the calibration files (io.py:8-245), and the
-covariance of a calibration (``calibration_covariance``: what a reference user derives from ``result.jac``).
+reprojection-error check of its result (viz.py:70-210) and the calibration files (io.py:8-245), the
+covariance of a calibration (``calibration_covariance``: what a reference user derives from ``result.jac``), and
+the least-squares refinement of triangulated points (``refine_points``).
 """
 from .geometry import (rodrigues, rodrigues_inv, rigid_transform_from_correspondences,
                        apply_rigid_transform, get_transformation_matrix, get_transformation_vector,
                        get_projection_matrix, euclidean_to_homogenous, homogeneous_to_euclidean,
-                       project_points, project_points_multi, undistort_points, triangulate)
+                       project_points, project_points_multi, undistort_points, triangulate,
+                       refine_points, RefinedPoints)
 from .bundle_adjustment import (embed_calib_objpoints, predict_calib_uvs, residuals,
                                 bundle_adjustment_sparsity, serialize_params, deserialize_params,
                                 bundle_adjust, select_frames)

@@ -45,6 +45,16 @@ class Result(ctypes.Structure):
                 ("status", ctypes.c_int32), ("kernel_launches", ctypes.c_int64)]
 
 
+# include/mcba.h MCBA_REFINE_LOSS_*: refine_points' own codes (scipy's five losses)
+REFINE_LOSSES = {"linear": 0, "soft_l1": 1, "huber": 2, "cauchy": 3, "arctan": 4}
+
+
+class RefineOptions(ctypes.Structure):
+    _fields_ = [("loss", ctypes.c_int32), ("f_scale", ctypes.c_double), ("sigma", ctypes.c_double),
+                ("ftol", ctypes.c_double), ("xtol", ctypes.c_double), ("gtol", ctypes.c_double),
+                ("max_iter", ctypes.c_int32), ("flags", ctypes.c_int32)]
+
+
 class McbaError(RuntimeError):
     def __init__(self, code, message):
         super().__init__(f"libmcba error {code}: {message}")
@@ -86,6 +96,8 @@ _SIGNATURES = {
     "mcba_embed_points": (_I, [_I, _P, _P, _L, _P, _I, _P]),
     "mcba_undistort_points": (_I, [_I, _P, _P, _L, _P, _P, _P]),
     "mcba_triangulate": (_I, [_I, _P, _P, _I, _L, _P, _P, _P, _P]),
+    "mcba_refine_points": (_I, [_I, _P, _P, _I, _L, _P, _P, _P, _P, ctypes.POINTER(RefineOptions),
+                                _P, _P, _P, _P, _P, _P, _P, _P]),
     "mcba_kernel_launches": (_L, [_P]),
     "mcba_plan_info": (_I, [_P, ctypes.POINTER(_L), _I]),
     "mcba_profile": (_I, [_P, _I, ctypes.POINTER(_D), ctypes.POINTER(_I)]),

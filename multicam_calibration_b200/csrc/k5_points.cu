@@ -346,7 +346,7 @@ __global__ void __launch_bounds__(128) triangulate_kernel(const double* __restri
   }
 }
 
-static void host_rodrigues(const double r[3], double R[9]) {
+void host_rodrigues(const double r[3], double R[9]) {
   const double th = std::sqrt(r[0] * r[0] + r[1] * r[1] + r[2] * r[2]);
   const double inv = th == 0.0 ? 1.0 : 1.0 / th;
   const double k[3] = {r[0] * inv, r[1] * inv, r[2] * inv};

@@ -172,6 +172,7 @@ struct EventPair {
 };
 
 int keep_async_pool(int device);   // k0_frontend.cu
+void host_rodrigues(const double r[3], double R[9]);   // k5_points.cu
 int peer_allreduce(mcba_handle* h, double* buf, long long n);   // mcba_peer.cu
 
 // kernel launchers (defined in the .cu files)

@@ -7,6 +7,7 @@ helpers (a handful of 3x3 / 4x4 operations the reference calls once per camera
 or frame) are host numpy, as SURVEY.md section 2 scopes them.
 """
 import ctypes
+from typing import NamedTuple, Optional
 
 import numpy as np
 
@@ -196,3 +197,127 @@ def triangulate(all_uvs, all_extrinsics, all_intrinsics):
     check(lib.mcba_triangulate(dev, stream, ctypes.c_void_p(d_uv.data_ptr()), C, P, _h(ext), _h(Ks),
                                _h(dists), ctypes.c_void_p(d_out.data_ptr())))
     return _native.to_host(d_out)
+
+
+class RefinedPoints(NamedTuple):
+    """Result of :func:`refine_points`; per-point arrays over the P points."""
+    points: np.ndarray        # (P, 3) refined points
+    cost: np.ndarray          # (P,) 0.5 sum rho at the result
+    rms: np.ndarray           # (P,) reprojection RMS in px over the point's finite scalars
+    n_views: np.ndarray       # (P,) int, seen views
+    status: np.ndarray        # (P,) int8: 1 gtol, 2 ftol, 3 xtol, 4 ftol + xtol, 0 max_iter, -1, -2
+    iterations: np.ndarray    # (P,) int16, trial steps
+    covariance: Optional[np.ndarray]    # (P, 3, 3) or None
+    view_errors: Optional[np.ndarray]   # (C, P) px, NaN where unseen, or None
+
+
+def _real_array(name, a):
+    a = np.asarray(a)
+    if not (np.issubdtype(a.dtype, np.floating) or np.issubdtype(a.dtype, np.integer)):
+        raise ValueError(f"refine_points: {name} must be a real array, got dtype {a.dtype}")
+    return np.ascontiguousarray(a, dtype=np.float64)
+
+
+def _positive(name, v):
+    if isinstance(v, (bool, np.bool_)) or not isinstance(v, (int, float, np.integer, np.floating)) \
+            or not (0 < float(v) < np.inf):
+        raise ValueError(f"refine_points: {name} must be a finite number > 0, got {v!r}")
+    return float(v)
+
+
+def refine_points(all_uvs, all_extrinsics, all_intrinsics, points=None, *, loss="linear", f_scale=1.0, sigma=1.0,
+                  max_iter=50, ftol=1e-12, xtol=1e-12, gtol=1e-10, covariance=True, view_errors=False):
+    """Least-squares refinement of triangulated points on the device (``mcba_refine_points``).
+
+    Per point, Levenberg-Marquardt on ``0.5 sum_views sum_{u,v} f_scale^2 rho((r / f_scale)^2)`` with
+    ``r = observed - project_points(X, ext_c, K_c, dist_c)``: the model of ``project_points`` and the bundle
+    adjustment (full K with skew, k1 and k2 only).  ``loss`` is one of scipy's ``linear``, ``soft_l1``,
+    ``huber``, ``cauchy``, ``arctan`` with scipy's formulas and ``f_scale``; the ftol / xtol / gtol tests are
+    scipy's (``least_squares``), applied per point.
+
+    Inputs are ``triangulate``'s: ``all_uvs`` a list of C ``(P, 2)`` arrays or a ``(C, P, 2)`` array, NaN
+    marking a missing view; a view whose pixel does not undistort to a finite point (NaN, +-inf, an
+    overflowing value) is unseen, as in ``triangulate``.  ``points=None`` starts from ``triangulate``'s
+    result, computed in the same device call; a given ``(P, 3)`` start is used as is.  The start's
+    triangulation undistorts with all five coefficients of ``dist`` while the objective uses k1, k2 only: with
+    non-zero p1, p2 or k3 the two models disagree and the refined point minimises the two-coefficient one.
+
+    A view behind a camera at the start still enters the objective as ``project_points`` evaluates it
+    (through the camera centre).  Status per point: 1 gtol, 2 ftol, 3 xtol, 4 ftol and xtol, 0 ``max_iter``
+    trial steps reached (the point is refined in all of these); -1 fewer than two seen views (NaN point, as
+    ``triangulate`` gives); -2 a non-finite start or cost at the start (a view on a camera's Z = 0 plane), or
+    damping beyond its bound: the start is returned unchanged.  ``covariance`` is
+    ``sigma^2 inv(J~^T J~)`` at the result with ``J~`` scaled for the robust loss as scipy's ``result.jac``.
+    """
+    if callable(loss) or not isinstance(loss, str) or loss not in _native.REFINE_LOSSES:
+        raise ValueError(f"refine_points: loss must be one of {sorted(_native.REFINE_LOSSES)}, got {loss!r}")
+    f_scale = _positive("f_scale", f_scale)
+    sigma = _positive("sigma", sigma)
+    if isinstance(max_iter, (bool, np.bool_)) or not isinstance(max_iter, (int, np.integer)) \
+            or not 1 <= max_iter <= 32767:
+        raise ValueError(f"refine_points: max_iter must be an integer in [1, 32767], got {max_iter!r}")
+    tols = {}
+    for name, v in (("ftol", ftol), ("xtol", xtol), ("gtol", gtol)):
+        if isinstance(v, (bool, np.bool_)) or not isinstance(v, (int, float, np.integer, np.floating)) \
+                or not (0 <= float(v) < np.inf):
+            raise ValueError(f"refine_points: {name} must be a finite number >= 0, got {v!r}")
+        tols[name] = float(v)
+    if isinstance(all_uvs, np.ndarray):
+        uv = _real_array("all_uvs", all_uvs)
+    else:
+        uv = np.stack([_real_array("all_uvs", u) for u in all_uvs]) if len(all_uvs) else np.zeros((0, 0, 2))
+    if uv.ndim != 3 or uv.shape[2] != 2:
+        raise ValueError(f"refine_points: all_uvs must be C arrays (P, 2) or one (C, P, 2) array, got {uv.shape}")
+    C, P, _ = uv.shape
+    if not 1 <= C <= 32:
+        raise ValueError(f"refine_points: 1 <= n_cameras <= 32, got {C}")
+    ext = _real_array("all_extrinsics", all_extrinsics)
+    if ext.shape != (C, 6):
+        raise ValueError(f"refine_points: all_extrinsics must be ({C}, 6), got {ext.shape}")
+    if len(all_intrinsics) != C:
+        raise ValueError(f"refine_points: all_intrinsics must have {C} entries, got {len(all_intrinsics)}")
+    Ks = np.empty((C, 3, 3))
+    dists = np.zeros((C, 5))
+    for c, intr in enumerate(all_intrinsics):
+        if len(intr) != 2:
+            raise ValueError("refine_points: all_intrinsics entries must be (camera_matrix, dist_coefs)")
+        K = _real_array("camera_matrix", intr[0])
+        dc = _real_array("dist_coefs", intr[1]).ravel()
+        if K.shape != (3, 3) or not 2 <= dc.size:
+            raise ValueError(f"refine_points: camera {c}: camera_matrix must be (3, 3) and dist_coefs hold at "
+                             f"least k1, k2, got {K.shape} and {dc.size} coefficients")
+        Ks[c] = K
+        dists[c, :min(dc.size, 5)] = dc[:5]
+    init = None
+    if points is not None:
+        init = _real_array("points", points)
+        if init.shape != (P, 3):
+            raise ValueError(f"refine_points: points must be ({P}, 3), got {init.shape}")
+
+    torch, lib, dev = _device_ctx()
+    d_uv = _native.to_device(uv, dev)
+    d_init = None if init is None else _native.to_device(init, dev)
+    f64 = dict(dtype=torch.float64, device=d_uv.device)
+    d_pts = torch.empty((P, 3), **f64)
+    d_cost = torch.empty((P,), **f64)
+    d_rms = torch.empty((P,), **f64)
+    d_status = torch.empty((P,), dtype=torch.int8, device=d_uv.device)
+    d_iters = torch.empty((P,), dtype=torch.int16, device=d_uv.device)
+    d_nv = torch.empty((P,), dtype=torch.int8, device=d_uv.device)
+    d_cov = torch.empty((P, 6), **f64) if covariance else None
+    d_verr = torch.empty((C, P), **f64) if view_errors else None
+    opt = _native.RefineOptions(loss=_native.REFINE_LOSSES[loss], f_scale=f_scale, sigma=sigma,
+                                max_iter=int(max_iter), flags=0, **tols)
+
+    def ptr(t):
+        return None if t is None else ctypes.c_void_p(t.data_ptr())
+    stream = ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+    check(lib.mcba_refine_points(dev, stream, ptr(d_uv), C, P, _h(ext), _h(Ks), _h(dists), ptr(d_init),
+                                 ctypes.byref(opt), ptr(d_pts), ptr(d_cost), ptr(d_rms), ptr(d_status),
+                                 ptr(d_iters), ptr(d_cov), ptr(d_verr), ptr(d_nv)))
+    cov = None
+    if covariance:
+        cov = _native.to_host(d_cov)[:, [0, 1, 2, 1, 3, 4, 2, 4, 5]].reshape(P, 3, 3)
+    return RefinedPoints(_native.to_host(d_pts), _native.to_host(d_cost), _native.to_host(d_rms),
+                         _native.to_host(d_nv).astype(np.int64), _native.to_host(d_status),
+                         _native.to_host(d_iters), cov, _native.to_host(d_verr) if view_errors else None)
