@@ -312,6 +312,20 @@ int mcba_refine_points(int device, void* cuda_stream, const double* d_uvs, int n
                        const mcba_refine_options* opt, double* d_points, double* d_cost, double* d_rms,
                        int8_t* d_status, int16_t* d_iters, double* d_cov, double* d_view_err, int8_t* d_n_views);
 
+/* Calibration uncertainty carried into refined points (covariance.point_covariance).  At each point X (d_points,
+ * e.g. mcba_refine_points' result) and over its seen views V (the rule above), with J~ scaled as d_cov of
+ * mcba_refine_points (same loss, f_scale):  H = J~_X^T J~_X,  S_c = -H^-1 J~_X^T J~_c (3 x 12, dX/dtheta_c, J~_c
+ * w.r.t. camera c's [fx fy cx cy k1 k2 rvec tvec]; skew held),  d_cov_meas = sigma^2 H^-1 (bit-identical to
+ * d_cov of mcba_refine_points at the same point),  d_cov_cal = sum_{c,d in V} S_c cov[c,d] S_d^T with h_cam_cov the
+ * (12C, 12C) row-major camera covariance (mcba_covariance's gauge).  Outputs (P,6) upper triangle xx xy xz yy yz
+ * zz; d_sens (P,3,12C) S with zero columns for unseen cameras (may be NULL); d_cov_meas may be NULL.  NaN where a
+ * point has fewer than two seen views, a non-finite X or a non-positive-definite H; d_cov_cal also NaN where a
+ * (c,d) block of h_cam_cov with c, d in V holds a non-finite entry.  loss MCBA_REFINE_LOSS_*, 1 <= C <= 32. */
+int mcba_point_covariance(int device, void* cuda_stream, const double* d_uvs, int n_cameras, int64_t n_points,
+                          const double* h_ext, const double* h_K, const double* h_dist, const double* d_points,
+                          const double* h_cam_cov, int loss, double f_scale, double sigma, double* d_cov_meas,
+                          double* d_cov_cal, double* d_sens);
+
 /* ---- reprojection-error QC (the step after bundle_adjust; viz.py:155-177 plot_residuals) ----
  * Per camera and frame whose N corners were all detected: undistort the detections (geometry.py:328-358),
  * homography detections -> board plane as cv2.findHomography computes it (float32-rounded points,

@@ -23,6 +23,6 @@ from .calibration import (estimate_pairwise_camera_transform, get_camera_spannin
 from .io import save_calibration, load_calibration
 from .viz import plot_residuals, reprojection_residuals
 from .engine import BAProblem, OptimizeResult
-from .covariance import calibration_covariance, CalibrationCovariance
+from .covariance import calibration_covariance, CalibrationCovariance, point_covariance, PointCovariance
 
 __version__ = "0.1.0"

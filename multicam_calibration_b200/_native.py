@@ -98,6 +98,7 @@ _SIGNATURES = {
     "mcba_triangulate": (_I, [_I, _P, _P, _I, _L, _P, _P, _P, _P]),
     "mcba_refine_points": (_I, [_I, _P, _P, _I, _L, _P, _P, _P, _P, ctypes.POINTER(RefineOptions),
                                 _P, _P, _P, _P, _P, _P, _P, _P]),
+    "mcba_point_covariance": (_I, [_I, _P, _P, _I, _L, _P, _P, _P, _P, _P, _I, _D, _D, _P, _P, _P]),
     "mcba_kernel_launches": (_L, [_P]),
     "mcba_plan_info": (_I, [_P, ctypes.POINTER(_L), _I]),
     "mcba_profile": (_I, [_P, _I, ctypes.POINTER(_D), ctypes.POINTER(_I)]),

@@ -6,6 +6,7 @@ engine never materialises J~ (16.8 M x 300 k at 6 cameras x 50,000 frames); :fun
 computes the same quantity from the reduced camera system and the per-frame factors of one device evaluation
 (``mcba_covariance``).
 """
+import ctypes
 from dataclasses import dataclass
 from typing import Optional
 
@@ -99,3 +100,96 @@ def calibration_covariance(all_calib_uvs, all_extrinsics, all_intrinsics, calib_
         camera=cam, camera_std=_std(np.diag(cam)).reshape(C, 12),
         poses=pose, pose_std=None if pose is None else _std(np.einsum("fii->fi", pose)),
         sigma2=info["sigma2"], dof=info["dof"], n_residuals=info["n_residuals"], cost=info["cost"])
+
+
+@dataclass
+class PointCovariance:
+    """``total = measurement + calibration`` (P, 3, 3) each: the uncertainty of refined points from the pixel
+    noise of their own observations and from the calibration; ``sensitivity`` (P, 3, 12C) ``dX/dtheta`` in the
+    order of ``serialize_params``, zero for unseen cameras, or None."""
+    total: np.ndarray
+    measurement: np.ndarray
+    calibration: np.ndarray
+    sensitivity: Optional[np.ndarray]
+
+
+def _camera_covariance(cov, C):
+    a = cov.camera if isinstance(cov, CalibrationCovariance) else cov
+    a = np.asarray(a)
+    if not (np.issubdtype(a.dtype, np.floating) or np.issubdtype(a.dtype, np.integer)):
+        raise ValueError(f"point_covariance: cov must be a CalibrationCovariance or a real array, got dtype {a.dtype}")
+    a = np.ascontiguousarray(a, dtype=np.float64)
+    n = 12 * C
+    if a.shape != (n, n):
+        raise ValueError(f"point_covariance: the camera covariance must be ({n}, {n}) for {C} cameras, got {a.shape}")
+    if np.isinf(a).any():
+        raise ValueError("point_covariance: the camera covariance must hold finite numbers or NaN")
+    nan = np.isnan(a)
+    if not np.array_equal(nan, nan.T):
+        raise ValueError("point_covariance: the camera covariance is not symmetric (NaN pattern)")
+    d = np.diag(a)
+    if (d < 0).any():
+        raise ValueError("point_covariance: the camera covariance has a negative diagonal entry")
+    with np.errstate(invalid="ignore"):
+        scale = np.sqrt(np.outer(d, d))
+        asym = np.abs(a - a.T) > 1e-9 * scale + 1e-300
+    if asym.any():
+        raise ValueError("point_covariance: the camera covariance is not symmetric")
+    return a
+
+
+def point_covariance(all_uvs, all_extrinsics, all_intrinsics, points, cov, loss="linear", f_scale=1.0, sigma=1.0,
+                     sensitivity=False):
+    """Covariance of refined points including the calibration's uncertainty (``mcba_point_covariance``).
+
+    ``all_uvs``, ``all_extrinsics``, ``all_intrinsics``, ``loss``, ``f_scale`` and ``sigma`` are taken as
+    ``refine_points`` takes them; ``points`` (P, 3) are the points to evaluate, normally ``refine_points(...).points``;
+    ``cov`` is a :class:`CalibrationCovariance` or its (12C, 12C) ``camera`` array.  Per point X over its seen
+    views, with J~ scaled as ``refine_points``' covariance scales it:
+
+    * ``measurement = sigma^2 inv(J~_X^T J~_X)``, bit-identical to ``refine_points(...).covariance`` at X;
+    * ``S_c = -inv(J~_X^T J~_X) J~_X^T J~_c`` (3 x 12), the Gauss-Newton sensitivity dX/dtheta_c of the minimiser
+      to camera c's parameters;
+    * ``calibration = sum_{c,d seen} S_c cov[c,d] S_d^T`` and ``total = measurement + calibration`` (the keypoint's
+      pixel noise is independent of the calibration data).
+
+    The calibration part is in the gauge of ``cov``: the reference camera's frame, or that of the camera pinned by
+    ``fixed=``.  Held parameters have zero rows and contribute nothing; unseen cameras do not enter.  A point
+    with fewer than two seen views, a non-finite X or a non-positive-definite J~_X^T J~_X is NaN in every output;
+    where a seen pair of cameras has NaN in its block of ``cov`` (a camera without observations in the
+    calibration), ``calibration`` and ``total`` are NaN.  For robust losses this is the Gauss-Newton recipe of
+    ``refine_points``' covariance, not a sandwich estimator.
+
+    ``sensitivity=True`` also returns S as (P, 3, 12C), zero for unseen cameras: ``S_i cov S_j^T`` is the
+    cross-covariance of points i and j (e.g. for the uncertainty of a distance between two keypoints).  It is
+    8 * 36 C bytes per point (1.7 GB at 1 M points and 6 cameras).
+    """
+    from . import _native
+    from .geometry import _device_ctx, _h, _loss_args, _real_array, _rig_args, check
+    who = "point_covariance"
+    loss_code, f_scale, sigma = _loss_args(loss, f_scale, sigma, who)
+    uv, ext, Ks, dists = _rig_args(all_uvs, all_extrinsics, all_intrinsics, who)
+    C, P, _ = uv.shape
+    X = _real_array("points", points, who)
+    if X.shape != (P, 3):
+        raise ValueError(f"{who}: points must be ({P}, 3), got {X.shape}")
+    cam = _camera_covariance(cov, C)
+
+    torch, lib, dev = _device_ctx()
+    d_uv = _native.to_device(uv, dev)
+    d_X = _native.to_device(X, dev)
+    f64 = dict(dtype=torch.float64, device=d_uv.device)
+    d_meas = torch.empty((P, 6), **f64)
+    d_cal = torch.empty((P, 6), **f64)
+    d_sens = torch.empty((P, 3, 12 * C), **f64) if sensitivity else None
+
+    def ptr(t):
+        return None if t is None or t.numel() == 0 else ctypes.c_void_p(t.data_ptr())
+    stream = ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+    check(lib.mcba_point_covariance(dev, stream, ptr(d_uv), C, P, _h(ext), _h(Ks), _h(dists), ptr(d_X), _h(cam),
+                                    loss_code, f_scale, sigma, ptr(d_meas), ptr(d_cal), ptr(d_sens)))
+    full = [0, 1, 2, 1, 3, 4, 2, 4, 5]
+    meas = _native.to_host(d_meas)[:, full].reshape(P, 3, 3)
+    cal = _native.to_host(d_cal)[:, full].reshape(P, 3, 3)
+    return PointCovariance(total=meas + cal, measurement=meas, calibration=cal,
+                           sensitivity=_native.to_host(d_sens) if sensitivity else None)

@@ -211,18 +211,56 @@ class RefinedPoints(NamedTuple):
     view_errors: Optional[np.ndarray]   # (C, P) px, NaN where unseen, or None
 
 
-def _real_array(name, a):
+def _real_array(name, a, who="refine_points"):
     a = np.asarray(a)
     if not (np.issubdtype(a.dtype, np.floating) or np.issubdtype(a.dtype, np.integer)):
-        raise ValueError(f"refine_points: {name} must be a real array, got dtype {a.dtype}")
+        raise ValueError(f"{who}: {name} must be a real array, got dtype {a.dtype}")
     return np.ascontiguousarray(a, dtype=np.float64)
 
 
-def _positive(name, v):
+def _positive(name, v, who="refine_points"):
     if isinstance(v, (bool, np.bool_)) or not isinstance(v, (int, float, np.integer, np.floating)) \
             or not (0 < float(v) < np.inf):
-        raise ValueError(f"refine_points: {name} must be a finite number > 0, got {v!r}")
+        raise ValueError(f"{who}: {name} must be a finite number > 0, got {v!r}")
     return float(v)
+
+
+def _loss_args(loss, f_scale, sigma, who="refine_points"):
+    """Validated (loss code, f_scale, sigma) of refine_points and point_covariance."""
+    if callable(loss) or not isinstance(loss, str) or loss not in _native.REFINE_LOSSES:
+        raise ValueError(f"{who}: loss must be one of {sorted(_native.REFINE_LOSSES)}, got {loss!r}")
+    return _native.REFINE_LOSSES[loss], _positive("f_scale", f_scale, who), _positive("sigma", sigma, who)
+
+
+def _rig_args(all_uvs, all_extrinsics, all_intrinsics, who="refine_points"):
+    """Validated (uv (C,P,2), ext (C,6), Ks (C,3,3), dists (C,5)) of refine_points and point_covariance."""
+    if isinstance(all_uvs, np.ndarray):
+        uv = _real_array("all_uvs", all_uvs, who)
+    else:
+        uv = np.stack([_real_array("all_uvs", u, who) for u in all_uvs]) if len(all_uvs) else np.zeros((0, 0, 2))
+    if uv.ndim != 3 or uv.shape[2] != 2:
+        raise ValueError(f"{who}: all_uvs must be C arrays (P, 2) or one (C, P, 2) array, got {uv.shape}")
+    C, P, _ = uv.shape
+    if not 1 <= C <= 32:
+        raise ValueError(f"{who}: 1 <= n_cameras <= 32, got {C}")
+    ext = _real_array("all_extrinsics", all_extrinsics, who)
+    if ext.shape != (C, 6):
+        raise ValueError(f"{who}: all_extrinsics must be ({C}, 6), got {ext.shape}")
+    if len(all_intrinsics) != C:
+        raise ValueError(f"{who}: all_intrinsics must have {C} entries, got {len(all_intrinsics)}")
+    Ks = np.empty((C, 3, 3))
+    dists = np.zeros((C, 5))
+    for c, intr in enumerate(all_intrinsics):
+        if len(intr) != 2:
+            raise ValueError(f"{who}: all_intrinsics entries must be (camera_matrix, dist_coefs)")
+        K = _real_array("camera_matrix", intr[0], who)
+        dc = _real_array("dist_coefs", intr[1], who).ravel()
+        if K.shape != (3, 3) or not 2 <= dc.size:
+            raise ValueError(f"{who}: camera {c}: camera_matrix must be (3, 3) and dist_coefs hold at "
+                             f"least k1, k2, got {K.shape} and {dc.size} coefficients")
+        Ks[c] = K
+        dists[c, :min(dc.size, 5)] = dc[:5]
+    return uv, ext, Ks, dists
 
 
 def refine_points(all_uvs, all_extrinsics, all_intrinsics, points=None, *, loss="linear", f_scale=1.0, sigma=1.0,
@@ -249,10 +287,7 @@ def refine_points(all_uvs, all_extrinsics, all_intrinsics, points=None, *, loss=
     damping beyond its bound: the start is returned unchanged.  ``covariance`` is
     ``sigma^2 inv(J~^T J~)`` at the result with ``J~`` scaled for the robust loss as scipy's ``result.jac``.
     """
-    if callable(loss) or not isinstance(loss, str) or loss not in _native.REFINE_LOSSES:
-        raise ValueError(f"refine_points: loss must be one of {sorted(_native.REFINE_LOSSES)}, got {loss!r}")
-    f_scale = _positive("f_scale", f_scale)
-    sigma = _positive("sigma", sigma)
+    loss_code, f_scale, sigma = _loss_args(loss, f_scale, sigma)
     if isinstance(max_iter, (bool, np.bool_)) or not isinstance(max_iter, (int, np.integer)) \
             or not 1 <= max_iter <= 32767:
         raise ValueError(f"refine_points: max_iter must be an integer in [1, 32767], got {max_iter!r}")
@@ -262,32 +297,8 @@ def refine_points(all_uvs, all_extrinsics, all_intrinsics, points=None, *, loss=
                 or not (0 <= float(v) < np.inf):
             raise ValueError(f"refine_points: {name} must be a finite number >= 0, got {v!r}")
         tols[name] = float(v)
-    if isinstance(all_uvs, np.ndarray):
-        uv = _real_array("all_uvs", all_uvs)
-    else:
-        uv = np.stack([_real_array("all_uvs", u) for u in all_uvs]) if len(all_uvs) else np.zeros((0, 0, 2))
-    if uv.ndim != 3 or uv.shape[2] != 2:
-        raise ValueError(f"refine_points: all_uvs must be C arrays (P, 2) or one (C, P, 2) array, got {uv.shape}")
+    uv, ext, Ks, dists = _rig_args(all_uvs, all_extrinsics, all_intrinsics)
     C, P, _ = uv.shape
-    if not 1 <= C <= 32:
-        raise ValueError(f"refine_points: 1 <= n_cameras <= 32, got {C}")
-    ext = _real_array("all_extrinsics", all_extrinsics)
-    if ext.shape != (C, 6):
-        raise ValueError(f"refine_points: all_extrinsics must be ({C}, 6), got {ext.shape}")
-    if len(all_intrinsics) != C:
-        raise ValueError(f"refine_points: all_intrinsics must have {C} entries, got {len(all_intrinsics)}")
-    Ks = np.empty((C, 3, 3))
-    dists = np.zeros((C, 5))
-    for c, intr in enumerate(all_intrinsics):
-        if len(intr) != 2:
-            raise ValueError("refine_points: all_intrinsics entries must be (camera_matrix, dist_coefs)")
-        K = _real_array("camera_matrix", intr[0])
-        dc = _real_array("dist_coefs", intr[1]).ravel()
-        if K.shape != (3, 3) or not 2 <= dc.size:
-            raise ValueError(f"refine_points: camera {c}: camera_matrix must be (3, 3) and dist_coefs hold at "
-                             f"least k1, k2, got {K.shape} and {dc.size} coefficients")
-        Ks[c] = K
-        dists[c, :min(dc.size, 5)] = dc[:5]
     init = None
     if points is not None:
         init = _real_array("points", points)
@@ -306,7 +317,7 @@ def refine_points(all_uvs, all_extrinsics, all_intrinsics, points=None, *, loss=
     d_nv = torch.empty((P,), dtype=torch.int8, device=d_uv.device)
     d_cov = torch.empty((P, 6), **f64) if covariance else None
     d_verr = torch.empty((C, P), **f64) if view_errors else None
-    opt = _native.RefineOptions(loss=_native.REFINE_LOSSES[loss], f_scale=f_scale, sigma=sigma,
+    opt = _native.RefineOptions(loss=loss_code, f_scale=f_scale, sigma=sigma,
                                 max_iter=int(max_iter), flags=0, **tols)
 
     def ptr(t):
