@@ -364,10 +364,10 @@ int64_t mcba_kernel_launches(mcba_handle* h);
 
 /* Kernel variants the handle's evaluation and solve take for its shape and observations (the launch
  * heuristics' choices, for tests that must show which branches they reached).  out[n] receives, at the
- * indices below: K2p warps per CTA and grid; K2c mode (0 general, 1 staged ring, 2 streamed pair),
- * warps of the streamed pair (0 otherwise) and its per-CTA partial count; SYRK warps, CTA rows (gy) and
- * the block count of its compiled tile list (0: listed at run time); the reduced solve (0 cuSOLVER,
- * 3 / 8 / 19 register tiles per warp, 119 = 19 tiles with the trailing ones in shared memory); frame
+ * indices below: K2p warps per CTA and grid; K2c mode (1 staged ring, 2 streamed pair), warps of the
+ * streamed pair (0 otherwise) and its per-CTA partial count; SYRK warps, CTA rows (gy) and the block
+ * count of its compiled tile list (0: listed at run time); the reduced solve (0 cuSOLVER, 3 / 8 register
+ * tiles per warp, 119 = 19 tiles per warp with the trailing ones in shared memory); frame
  * tiles; back-substitution grid; C; then the live (tile, camera) units of every camera (C entries).
  * n must be at least MCBA_PLAN_UNITS + C.  Synchronises the handle's stream. */
 #define MCBA_PLAN_K2P_WARPS 0

@@ -21,8 +21,8 @@ HESSIANS = {"auto": 0, "triggs": 1, "irls": 2}
 # mcba_plan_info: indices of the launch choices (include/mcba.h MCBA_PLAN_*); the live units per camera follow
 PLAN_FIELDS = ("k2p_warps", "k2p_grid", "k2c_mode", "k2c_warps", "k2c_parts", "syrk_warps", "syrk_gy",
                "syrk_static_nb", "solve", "tiles", "backsub_grid", "cameras")
-K2C_MODES = {0: "general", 1: "ring", 2: "stream"}
-SOLVE_TIERS = {0: "cusolver", 3: "regs3", 8: "regs8", 19: "regs19", 119: "smem19"}
+K2C_MODES = {1: "ring", 2: "stream"}
+SOLVE_TIERS = {0: "cusolver", 3: "regs3", 8: "regs8", 119: "smem19"}
 
 ITER_CALLBACK = ctypes.CFUNCTYPE(None, ctypes.c_void_p, ctypes.c_int, ctypes.c_int, ctypes.c_double,
                                  ctypes.c_double, ctypes.c_double, ctypes.c_double)

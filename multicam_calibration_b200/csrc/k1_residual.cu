@@ -4,7 +4,6 @@
 #include <cub/device/device_radix_sort.cuh>
 #include <cub/device/device_scan.cuh>
 
-#include <cstdlib>
 #include <type_traits>
 
 #include "mcba_internal.h"
@@ -158,56 +157,26 @@ __global__ void __launch_bounds__(256) tile_observations_kernel(const double2* _
   if ((threadIdx.x & 31) == 0 && finite) atomicAdd(n_scalars, (unsigned long long)finite);
 }
 
-// finite scalars per group of 32 consecutive (c,f,n) slots (one warp per group) + number of
-// observed corners: the exclusive scan of these counts positions every group of the compacted
-// residual vector (bundle_adjustment.py:97) without any per-row structure
-__global__ void count_groups_kernel(const double2* __restrict__ ref, long long slots, long long groups,
-                                    long long* __restrict__ counts, unsigned long long* __restrict__ n_obs) {
-  const int lane = threadIdx.x & 31;
-  const long long warp = (blockIdx.x * (long long)blockDim.x + threadIdx.x) >> 5;
-  const long long nwarps = ((long long)gridDim.x * blockDim.x) >> 5;
-  unsigned long long obs = 0;
-  for (long long g = warp; g < groups; g += nwarps) {
-    const long long i = g * 32 + lane;
-    bool fu = false, fv = false;
-    if (i < slots) {
-      const double2 o = ref[i];
-      fu = o.x == o.x;
-      fv = o.y == o.y;
-    }
-    const unsigned bu = __ballot_sync(0xffffffffu, fu), bv = __ballot_sync(0xffffffffu, fv);
-    if (lane == 0) {
-      counts[g] = __popc(bu) + __popc(bv);
-      obs += __popc(bu | bv);
-    }
-  }
-  if (lane == 0 && obs) atomicAdd(n_obs, obs);
-}
-
 int launch_tile_observations(mcba_handle* h) {
   const Layout& L = h->L;
   const int blocks = 148 * 8;
-  // ---- frame order: identity, or sorted by visibility mask
+  // ---- frame order: sorted by visibility mask.  The 32 frames of a tile share the leading ~log2(nTiles) bits of
+  //      the sorted key: all cameras when 2^C <= nTiles, the highest-numbered ones otherwise
   frame_mask_kernel<<<blocks, 256, 0, h->stream>>>(h->d_obs_ref, L.C, L.F, L.N, h->d_mask);
   iota_kernel<<<blocks, 256, 0, h->stream>>>(h->d_perm, L.Fpad);
-  h->launches += 2;
-  static const bool no_sort = getenv("MCBA_NO_FRAME_SORT") != nullptr;
-  if (!no_sort) {   // the 32 frames of a tile share the leading ~log2(nTiles) bits of the sorted key: all cameras
-                    // when 2^C <= nTiles, the highest-numbered ones otherwise
-    size_t bytes = 0;
-    unsigned int* keys_out = h->d_mask + L.Fpad;
-    int* vals_out = h->d_perm + L.Fpad;
-    cub::DeviceRadixSort::SortPairs(nullptr, bytes, h->d_mask, keys_out, h->d_perm, vals_out, (int)L.F, 0, L.C, h->stream);
-    if (bytes > h->sort_tmp_bytes) {
-      if (h->d_sort_tmp) cudaFree(h->d_sort_tmp);
-      MCBA_CUDA(cudaMalloc(&h->d_sort_tmp, bytes));
-      h->sort_tmp_bytes = bytes;
-    }
-    MCBA_CUDA(cub::DeviceRadixSort::SortPairs(h->d_sort_tmp, bytes, h->d_mask, keys_out, h->d_perm, vals_out, (int)L.F,
-                                              0, L.C, h->stream));
-    MCBA_CUDA(cudaMemcpyAsync(h->d_perm, vals_out, sizeof(int) * L.F, cudaMemcpyDeviceToDevice, h->stream));
-    h->launches += 2;
+  size_t bytes = 0;
+  unsigned int* keys_out = h->d_mask + L.Fpad;
+  int* vals_out = h->d_perm + L.Fpad;
+  cub::DeviceRadixSort::SortPairs(nullptr, bytes, h->d_mask, keys_out, h->d_perm, vals_out, (int)L.F, 0, L.C, h->stream);
+  if (bytes > h->sort_tmp_bytes) {
+    if (h->d_sort_tmp) cudaFree(h->d_sort_tmp);
+    MCBA_CUDA(cudaMalloc(&h->d_sort_tmp, bytes));
+    h->sort_tmp_bytes = bytes;
   }
+  MCBA_CUDA(cub::DeviceRadixSort::SortPairs(h->d_sort_tmp, bytes, h->d_mask, keys_out, h->d_perm, vals_out, (int)L.F,
+                                            0, L.C, h->stream));
+  MCBA_CUDA(cudaMemcpyAsync(h->d_perm, vals_out, sizeof(int) * L.F, cudaMemcpyDeviceToDevice, h->stream));
+  h->launches += 4;
   tile_active_kernel<<<blocks, 256, 0, h->stream>>>(h->d_mask, h->d_perm, L.F, L.nTiles, h->d_active);
   const long long units = L.nTiles * L.C;
   const int grid = (int)(units < 148 * 8 ? units : 148 * 8);
@@ -231,15 +200,10 @@ int launch_tile_observations(mcba_handle* h) {
   return MCBA_OK;
 }
 
-// ---- chunked K1 path --------------------------------------------------------------------------
+// ---- K1: residuals and predictions by chunks ---------------------------------------------------
 // A chunk = one camera's 32 consecutive frames = ONE contiguous block of 32*N double2 in the
 // reference layout (C,F,N,2), for the observations as well as for the predictions.
 constexpr int kChunkFrames = 32;
-
-static bool k1_use_chunks() {
-  static const bool flat = getenv("MCBA_K1_FLAT") != nullptr;
-  return !flat;
-}
 
 // finite scalars of every chunk (one warp per chunk, coalesced) + number of observed corners
 __global__ void count_chunks_kernel(const double2* __restrict__ ref, int C, long long F, int N, long long nBlk,
@@ -275,29 +239,21 @@ __global__ void count_chunks_kernel(const double2* __restrict__ ref, int C, long
   if (lane == 0 && obs) atomicAdd(n_obs, obs);
 }
 
-// offsets of the NaN compaction (bundle_adjustment.py:97) per chunk (or per group of 32 slots on
-// the fallback path for very large boards); only K1 needs them
+// offsets of the NaN compaction (bundle_adjustment.py:97) per chunk; only K1 needs them
 int ensure_row_offsets(mcba_handle* h) {
   if (h->have_rows) return MCBA_OK;
   const Layout& L = h->L;
-  const bool chunks = k1_use_chunks();
-  const long long slots = (long long)L.C * L.F * L.N;
   const long long nBlk = (L.F + kChunkFrames - 1) / kChunkFrames;
-  const long long groups = chunks ? (long long)L.C * nBlk : (slots + 31) / 32;
+  const long long groups = (long long)L.C * nBlk;
   unsigned long long* d_nobs = nullptr;
   MCBA_CUDA(cudaMalloc(&d_nobs, sizeof(unsigned long long)));
   MCBA_CUDA(cudaMemsetAsync(d_nobs, 0, sizeof(unsigned long long), h->stream));
   MCBA_CUDA(cudaMemsetAsync(h->d_row_off, 0, sizeof(long long) * (groups + 1), h->stream));
   int grid = (int)((groups * 32 + 255) / 256 < 148 * 16 ? (groups * 32 + 255) / 256 : 148 * 16);
   if (grid < 1) grid = 1;
-  if (chunks) {
-    if (!h->d_chunk_rows) MCBA_CUDA(cudaMalloc((void**)&h->d_chunk_rows, sizeof(unsigned int) * (size_t)(groups + 1)));
-    count_chunks_kernel<<<grid, 256, 0, h->stream>>>(reinterpret_cast<const double2*>(h->d_obs_ref), L.C, L.F, L.N, nBlk,
-                                                    h->d_row_off, h->d_chunk_rows, d_nobs);
-  }
-  else
-    count_groups_kernel<<<grid, 256, 0, h->stream>>>(reinterpret_cast<const double2*>(h->d_obs_ref), slots, groups,
-                                                    h->d_row_off, d_nobs);
+  if (!h->d_chunk_rows) MCBA_CUDA(cudaMalloc((void**)&h->d_chunk_rows, sizeof(unsigned int) * (size_t)(groups + 1)));
+  count_chunks_kernel<<<grid, 256, 0, h->stream>>>(reinterpret_cast<const double2*>(h->d_obs_ref), L.C, L.F, L.N, nBlk,
+                                                  h->d_row_off, h->d_chunk_rows, d_nobs);
   h->launches++;
   MCBA_CUDA(cudaGetLastError());
   size_t tmp_bytes = 0;
@@ -330,8 +286,8 @@ int ensure_row_offsets(mcba_handle* h) {
 //            projection for both scalars, then either the ballot-compacted residuals in the
 //            reference's order c, f, n, {u, v} (bundle_adjustment.py:97) from a running offset
 //            that starts at the chunk's scanned offset, or the coalesced predictions.
-// Per group of 32 slots this is ~80 warp instructions (45 of them FP64) against ~160 for the
-// per-slot indexing of the fallback kernel below.
+// Per group of 32 slots this is ~80 warp instructions (45 of them FP64) against ~160 for a flat
+// kernel that indexes every (c,f,n) slot on its own.
 #ifndef MCBA_K1_CTAS
 #define MCBA_K1_CTAS 4
 #endif
@@ -490,153 +446,9 @@ static int launch_chunks(mcba_handle* h, const double* x, double* out, bool comp
   return MCBA_OK;
 }
 
-// K1 without the chunk structure (kept for comparison; MCBA_K1_FLAT=1 selects it).  Two passes:
-//   row_transforms_kernel  one thread per (c,f) row: the composed transform X_c = Rcf X_o + tcf
-//                          (Rodrigues once per row instead of once per lane), 96 B per row;
-//   residuals_kernel       one warp per 32 consecutive (c,f,n) slots: one coalesced double2 load
-//                          and ONE projection per corner for both scalars, ballot-prefix
-//                          compaction in the reference's order (c,f,n,{u,v})
-//                          (bundle_adjustment.py:97) from per-group offsets.
-__global__ void row_transforms_kernel(const double* __restrict__ x, const CamConst* __restrict__ cams, int C,
-                                      long long F, double* __restrict__ rowT /* [C*F][12] */) {
-  const long long row = blockIdx.x * (long long)blockDim.x + threadIdx.x;
-  if (row >= (long long)C * F) return;
-  const int c = (int)(row / F);
-  const long long f = row % F;
-  const CamConst& cam = cams[c];
-  const double* ps = x + 12 * (long long)C + 6 * f;
-  const double rho[3] = {ps[0], ps[1], ps[2]}, tau[3] = {ps[3], ps[4], ps[5]};
-  double Rp[9], Rcf[9], tcf[3];
-  rodrigues(rho, Rp);
-  mat3_mul(cam.R, Rp, Rcf);
-  mat3_vec(cam.R, tau, tcf);
-  double2* o = reinterpret_cast<double2*>(rowT + row * 12);
-  o[0] = make_double2(Rcf[0], Rcf[1]);
-  o[1] = make_double2(Rcf[2], Rcf[3]);
-  o[2] = make_double2(Rcf[4], Rcf[5]);
-  o[3] = make_double2(Rcf[6], Rcf[7]);
-  o[4] = make_double2(Rcf[8], tcf[0] + cam.t[0]);
-  o[5] = make_double2(tcf[1] + cam.t[1], tcf[2] + cam.t[2]);
-}
+int launch_residuals(mcba_handle* h, const double* x, double* r_out) { return launch_chunks(h, x, r_out, true); }
 
-// Idx: unsigned int while C*F*N < 2^32 (two 32-bit divisions per lane instead of two 64-bit ones,
-// which alone made the kernel instruction bound: 180 -> ~70 warp instructions per group).
-template <bool kCompact, typename Idx>
-__global__ void __launch_bounds__(256) residuals_kernel(const double* __restrict__ rowT, const double2* __restrict__ ref,
-                                                        const double* __restrict__ obj,
-                                                        const CamConst* __restrict__ cams,
-                                                        const long long* __restrict__ grp_off, int C, long long F,
-                                                        int N, long long slots, double* __restrict__ out) {
-  extern __shared__ double s_obj[];
-  for (int i = threadIdx.x; i < 3 * N; i += blockDim.x) s_obj[i] = obj[i];
-  __syncthreads();
-  const int lane = threadIdx.x & 31;
-  const long long warp = (blockIdx.x * (long long)blockDim.x + threadIdx.x) >> 5;
-  const long long nwarps = ((long long)gridDim.x * blockDim.x) >> 5;
-  const long long groups = (slots + 31) / 32;
-  constexpr int kU = 4;   // groups per warp iteration: four independent 512-byte loads in flight per warp
-  for (long long g0 = warp * kU; g0 < groups; g0 += nwarps * kU) {
-    double2 o[kU];
-    long long off[kU];
-#pragma unroll
-    for (int u = 0; u < kU; ++u) {
-      const long long i = (g0 + u) * 32 + lane;
-      o[u] = make_double2(0.0, 0.0);
-      off[u] = 0;
-      if (kCompact && i < slots) o[u] = ref[i];                       // coalesced: 512 contiguous bytes per warp
-      if (kCompact && g0 + u < groups) off[u] = grp_off[g0 + u];
-    }
-#pragma unroll
-    for (int u = 0; u < kU; ++u) {
-      const long long i = (g0 + u) * 32 + lane;
-      bool fu = false, fv = false;
-      double ru = 0.0, rv = 0.0;
-      if (i < slots) {
-        const Idx row = (Idx)i / (Idx)N;
-        const int n = (int)((Idx)i - row * (Idx)N);
-        const int c = (int)(row / (Idx)F);
-        const CamConst& cam = cams[c];
-        const Intr in{cam.fx, cam.fy, cam.cx, cam.cy, cam.k1, cam.k2};
-        const double2* t2 = reinterpret_cast<const double2*>(rowT + (size_t)row * 12);   // <= 2-3 distinct rows per warp
-        const double2 t0 = t2[0], t1 = t2[1], t2v = t2[2], t3 = t2[3], t4 = t2[4], t5 = t2[5];
-        const double Rcf[9] = {t0.x, t0.y, t1.x, t1.y, t2v.x, t2v.y, t3.x, t3.y, t4.x};
-        const double tcf[3] = {t4.y, t5.x, t5.y};
-        double pu, pv;
-        project(in, Rcf, tcf, s_obj[3 * n], s_obj[3 * n + 1], s_obj[3 * n + 2], pu, pv);
-        if (kCompact) {
-          fu = o[u].x == o[u].x;
-          fv = o[u].y == o[u].y;
-          ru = o[u].x - pu;
-          rv = o[u].y - pv;
-        } else {
-          reinterpret_cast<double2*>(out)[i] = make_double2(pu, pv);
-        }
-      }
-      if (kCompact) {
-        const unsigned bu = __ballot_sync(0xffffffffu, fu), bv = __ballot_sync(0xffffffffu, fv);
-        const unsigned lt = (1u << lane) - 1u;
-        const long long pos = off[u] + __popc(bu & lt) + __popc(bv & lt);
-        if (fu) out[pos] = ru;
-        if (fv) out[pos + (fu ? 1 : 0)] = rv;
-      }
-    }
-  }
-}
-
-static int rows_grid(long long rows) {
-  long long g = (rows * 32 + 255) / 256;
-  if (g > 148 * 16) g = 148 * 16;
-  if (g < 1) g = 1;
-  return (int)g;
-}
-
-static int launch_row_transforms(mcba_handle* h, const double* x) {
-  const Layout& L = h->L;
-  int rc = launch_prep_cameras(h, x);
-  if (rc) return rc;
-  const long long rows = (long long)L.C * L.F;
-  if (!h->d_rowT) MCBA_CUDA(cudaMalloc(&h->d_rowT, sizeof(double) * 12 * rows));   // K1 only: allocated on first use
-  row_transforms_kernel<<<(int)((rows + 255) / 256), 256, 0, h->stream>>>(x, h->d_cams, L.C, L.F, h->d_rowT);
-  h->launches++;
-  MCBA_CUDA(cudaGetLastError());
-  return MCBA_OK;
-}
-
-int launch_residuals(mcba_handle* h, const double* x, double* r_out) {
-  const Layout& L = h->L;
-  if (k1_use_chunks()) return launch_chunks(h, x, r_out, true);
-  int rc = launch_row_transforms(h, x);
-  if (rc) return rc;
-  const long long slots = (long long)L.C * L.F * L.N;
-  if (slots < (1ll << 32))
-    residuals_kernel<true, unsigned int><<<rows_grid((slots + 31) / 32), 256, sizeof(double) * 3 * L.N, h->stream>>>(
-        h->d_rowT, reinterpret_cast<const double2*>(h->d_obs_ref), h->d_obj, h->d_cams, h->d_row_off, L.C, L.F, L.N,
-        slots, r_out);
-  else
-    residuals_kernel<true, long long><<<rows_grid((slots + 31) / 32), 256, sizeof(double) * 3 * L.N, h->stream>>>(
-        h->d_rowT, reinterpret_cast<const double2*>(h->d_obs_ref), h->d_obj, h->d_cams, h->d_row_off, L.C, L.F, L.N,
-        slots, r_out);
-  h->launches++;
-  MCBA_CUDA(cudaGetLastError());
-  return MCBA_OK;
-}
-
-int launch_predict(mcba_handle* h, const double* x, double* uv_out) {
-  const Layout& L = h->L;
-  if (k1_use_chunks()) return launch_chunks(h, x, uv_out, false);
-  int rc = launch_row_transforms(h, x);
-  if (rc) return rc;
-  const long long slots = (long long)L.C * L.F * L.N;
-  if (slots < (1ll << 32))
-    residuals_kernel<false, unsigned int><<<rows_grid((slots + 31) / 32), 256, sizeof(double) * 3 * L.N, h->stream>>>(
-        h->d_rowT, nullptr, h->d_obj, h->d_cams, nullptr, L.C, L.F, L.N, slots, uv_out);
-  else
-    residuals_kernel<false, long long><<<rows_grid((slots + 31) / 32), 256, sizeof(double) * 3 * L.N, h->stream>>>(
-        h->d_rowT, nullptr, h->d_obj, h->d_cams, nullptr, L.C, L.F, L.N, slots, uv_out);
-  h->launches++;
-  MCBA_CUDA(cudaGetLastError());
-  return MCBA_OK;
-}
+int launch_predict(mcba_handle* h, const double* x, double* uv_out) { return launch_chunks(h, x, uv_out, false); }
 
 // ---------------------------------------------------------------- robust cost
 // warp per (tile, camera), lane = frame, tiled SoA (the walk of K2p without the Jacobian); C ABI mcba_cost

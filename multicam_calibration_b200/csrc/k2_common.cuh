@@ -5,6 +5,42 @@
 
 namespace mcba {
 
+// Bulk async copies into shared memory, completed on an mbarrier (K2c, SYRK, back-substitution).
+__device__ __forceinline__ unsigned smem_u32(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
+
+__device__ __forceinline__ void mbar_init(unsigned long long* bar, unsigned count) {
+  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
+}
+__device__ __forceinline__ void mbar_expect_tx(unsigned long long* bar, unsigned bytes) {
+  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
+}
+__device__ __forceinline__ void mbar_arrive(unsigned long long* bar) {
+  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
+}
+__device__ __forceinline__ void mbar_wait(unsigned long long* bar, unsigned parity) {
+  asm volatile(
+      "{\n"
+      ".reg .pred p;\n"
+      "WAIT_LOOP:\n"
+      "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
+      "@p bra WAIT_DONE;\n"
+      "bra WAIT_LOOP;\n"
+      "WAIT_DONE:\n"
+      "}\n" ::"r"(smem_u32(bar)), "r"(parity) : "memory");
+}
+__device__ __forceinline__ void tma_load_1d(void* dst, const void* src, unsigned bytes, unsigned long long* bar) {
+  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(smem_u32(dst)),
+               "l"(src), "r"(bytes), "r"(smem_u32(bar))
+               : "memory");
+}
+
+// FP64 tensor path: C (8 x 8, two values per lane) += A (8 x 4) B (4 x 8), one value of each per lane (SYRK, solve).
+__device__ __forceinline__ void dmma_m8n8k4(double& c0, double& c1, double a, double b) {
+  asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};"
+               : "+d"(c0), "+d"(c1)
+               : "d"(a), "d"(b));
+}
+
 __host__ __device__ constexpr int tri12(int i, int j) { return i * 12 - (i * (i - 1)) / 2 + (j - i); }
 __host__ __device__ constexpr int sym12(int i, int j) { return i <= j ? tri12(i, j) : tri12(j, i); }
 __host__ __device__ constexpr int tri6(int i, int j) { return i * 6 - (i * (i - 1)) / 2 + (j - i); }

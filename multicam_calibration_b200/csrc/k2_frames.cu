@@ -12,11 +12,9 @@
 //       (lane = frame is the fastest index of H, Z, y, L^-1).  HBM bound: reads 504 B,
 //       writes 576 B per pair.
 //
-// K2c comes in three builds (k2_consumer_parts): the staged ring for 2-6 cameras, a streamed pair of kernels
-// (pose block per tile, Z rows per live unit) for any other count, and the plain general kernel as the fall-back.
+// K2c comes in two builds (k2_consumer_parts): the staged ring for 2-6 cameras and a streamed pair of kernels
+// (pose block per tile, Z rows per live unit) for any other count.
 // A rejected LM step only changes lambda: K2c is re-run on the same hand-off, K2p is not.
-#include <cstdlib>
-
 #include "k2_producer.cuh"
 
 namespace mcba {
@@ -169,72 +167,6 @@ __device__ __forceinline__ void store_pose_outputs(const K2CParams& p, long long
   }
 }
 
-// General path (any camera count): one CTA per frame tile, warp w handles cameras w, w + kW, ...
-// reading the hand-off from global memory; partial outputs per tile.
-template <int kW>
-__global__ void __launch_bounds__(kW * 32, 2) k2c_kernel(const K2CParams p) {
-  __shared__ double s_V[kW][27][32];
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const int C = p.C, nc = 12 * C;
-  const long long tile = blockIdx.x;
-  const long long f = p.perm[tile * kTile + lane];
-  const bool fvalid = f >= 0;
-  double pose[6];
-#pragma unroll
-  for (int i = 0; i < 6; ++i) pose[i] = fvalid ? p.x[(size_t)nc + f * 6 + i] : 0.0;
-  double Jl[9];
-  so3_left_jacobian(pose, Jl);
-
-  double Vpp[21], gpp[6];
-#pragma unroll
-  for (int i = 0; i < 21; ++i) Vpp[i] = 0.0;
-#pragma unroll
-  for (int i = 0; i < 6; ++i) gpp[i] = 0.0;
-  for (int c = warp; c < C; c += kW) {
-    double Rc[9], K[9];
-    pose_map(p.cams[c], pose, Rc, K);
-    pose_block_add(p.H + ((size_t)(tile * C + c) * kHandoff) * kTile + lane, Rc, K, Vpp, gpp);
-  }
-  // exchange the partial sums (every warp then holds the full pose block; fixed order)
-  if (kW > 1) {
-#pragma unroll
-    for (int i = 0; i < 21; ++i) s_V[warp][i][lane] = Vpp[i];
-#pragma unroll
-    for (int i = 0; i < 6; ++i) s_V[warp][21 + i][lane] = gpp[i];
-    __syncthreads();
-#pragma unroll
-    for (int i = 0; i < 21; ++i) Vpp[i] = 0.0;
-#pragma unroll
-    for (int i = 0; i < 6; ++i) gpp[i] = 0.0;
-#pragma unroll
-    for (int w = 0; w < kW; ++w) {
-#pragma unroll
-      for (int i = 0; i < 21; ++i) Vpp[i] += s_V[w][i][lane];
-#pragma unroll
-      for (int i = 0; i < 6; ++i) gpp[i] += s_V[w][21 + i][lane];
-    }
-  }
-  double Linv[21], yv[6], gp[6], gmax = 0.0;
-  pose_block_factor(Vpp, gpp, Jl, p.lambda, p.D2pose + (size_t)tile * 6 * 32 + lane, warp == 0, Linv, yv, gp, gmax);
-  if (warp == 0) {
-    store_pose_outputs(p, tile, f, fvalid, lane, Linv, yv, gp);
-#pragma unroll
-    for (int off = 16; off >= 1; off >>= 1) gmax = fmax(gmax, __shfl_xor_sync(0xffffffffu, gmax, off));
-    if (lane == 0) p.partG[tile] = gmax;
-  }
-  for (int c = warp; c < C; c += kW) {
-    double Rc[9], K[9];
-    pose_map(p.cams[c], pose, Rc, K);
-    double zy[12];
-#pragma unroll
-    for (int i = 0; i < 12; ++i) zy[i] = 0.0;
-    z_rows(p.H + ((size_t)(tile * C + c) * kHandoff) * kTile + lane, Rc, K, Jl, Linv, yv,
-           p.Z + ((size_t)(tile * nc + c * 12) * 6) * kTile + lane, zy);
-    const double v = zy_lane_sum(zy, lane);
-    if (lane < 12) p.partZy[(size_t)tile * nc + c * 12 + lane] = v;
-  }
-}
-
 // Staged path (kC <= 6 cameras, warp = camera): persistent CTAs, two per SM.  The whole hand-off
 // block of a tile (kC x 63 x 32 doubles, contiguous) arrives by ONE bulk async copy into shared
 // memory; while one CTA of the SM waits for its copy the other one computes, so no warp waits on
@@ -242,19 +174,6 @@ __global__ void __launch_bounds__(kW * 32, 2) k2c_kernel(const K2CParams p) {
 // rows.  The cross-camera sum of the pose block goes through a small exchange buffer in two
 // rounds (11 + 10 values; g'' travels in the camera's already consumed q_ext slots of the
 // stage), which is what lets two CTAs fit in the 228 KB of an SM.  Partial outputs per CTA.
-__device__ __forceinline__ unsigned k2c_smem_u32(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void k2c_mbar_wait(unsigned long long* bar, unsigned parity) {
-  asm volatile(
-      "{\n"
-      ".reg .pred p;\n"
-      "K2C_WAIT_LOOP:\n"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-      "@p bra K2C_WAIT_DONE;\n"
-      "bra K2C_WAIT_LOOP;\n"
-      "K2C_WAIT_DONE:\n"
-      "}\n" ::"r"(k2c_smem_u32(bar)), "r"(parity) : "memory");
-}
-
 constexpr int kXchg = 11;   // values per exchange round
 
 template <int kC>
@@ -276,26 +195,20 @@ __global__ void __launch_bounds__(kC * 32, 2) k2c_ring_kernel(const K2CParams p)
     const unsigned m = p.active[tile] & ((1u << kC) - 1u);
     constexpr unsigned kUnitBytes = kHandoff * kTile * sizeof(double);
     const unsigned bytes = (unsigned)__popc(m) * kUnitBytes;
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(k2c_smem_u32(&full_bar)), "r"(bytes) : "memory");
+    mbar_expect_tx(&full_bar, bytes);
     if (m == (1u << kC) - 1u) {
-      asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                       k2c_smem_u32(stage)),
-                   "l"(p.H + (size_t)tile * kStage), "r"(bytes), "r"(k2c_smem_u32(&full_bar))
-                   : "memory");
+      tma_load_1d(stage, p.H + (size_t)tile * kStage, bytes, &full_bar);
     } else {
 #pragma unroll
       for (int cc = 0; cc < kC; ++cc) {
         if ((m >> cc) & 1u)
-          asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                           k2c_smem_u32(stage + (size_t)cc * kHandoff * kTile)),
-                       "l"(p.H + (size_t)tile * kStage + (size_t)cc * kHandoff * kTile), "r"(kUnitBytes),
-                       "r"(k2c_smem_u32(&full_bar))
-                       : "memory");
+          tma_load_1d(stage + (size_t)cc * kHandoff * kTile, p.H + (size_t)tile * kStage + (size_t)cc * kHandoff * kTile,
+                      kUnitBytes, &full_bar);
       }
     }
   };
   if (threadIdx.x == 0) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(k2c_smem_u32(&full_bar)));
+    mbar_init(&full_bar, 1);
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     if (n_it > 0) issue(0);
   }
@@ -317,7 +230,7 @@ __global__ void __launch_bounds__(kC * 32, 2) k2c_ring_kernel(const K2CParams p)
     double Jl[9], Rc[9], K[9];
     so3_left_jacobian(pose, Jl);
     pose_map(cam, pose, Rc, K);
-    k2c_mbar_wait(&full_bar, (unsigned)(it & 1));
+    mbar_wait(&full_bar, (unsigned)(it & 1));
     double Vpp[21], gpp[6];
     {
       double Vp[21], gq[6];
@@ -418,8 +331,8 @@ __device__ __forceinline__ K2cStreamShared k2c_stream_carve(unsigned char* smem_
 template <int kW>
 __device__ __forceinline__ void k2c_stream_init(const K2CParams& p, const K2cStreamShared& s, int lane) {
   if (lane == 0) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(k2c_smem_u32(s.bar)));
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(k2c_smem_u32(s.bar + 1)));
+    mbar_init(s.bar, 1);
+    mbar_init(s.bar + 1, 1);
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
   for (int i = threadIdx.x; i < p.C * 12; i += kW * 32) {
@@ -429,12 +342,9 @@ __device__ __forceinline__ void k2c_stream_init(const K2CParams& p, const K2cStr
   }
 }
 __device__ __forceinline__ void k2c_stream_copy(const K2cStreamShared& s, unsigned k, const double* src, unsigned rows) {
-  const unsigned b = k2c_smem_u32(s.bar + (k & 1u)), bytes = rows * kTile * (unsigned)sizeof(double);
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(b), "r"(bytes) : "memory");
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                   k2c_smem_u32(s.ring + (size_t)(k & 1u) * kStreamStage)),
-               "l"(src), "r"(bytes), "r"(b)
-               : "memory");
+  const unsigned bytes = rows * kTile * (unsigned)sizeof(double);
+  mbar_expect_tx(s.bar + (k & 1u), bytes);
+  tma_load_1d(s.ring + (size_t)(k & 1u) * kStreamStage, src, bytes, s.bar + (k & 1u));
 }
 // E' of camera c for this lane's pose from the shared copy of R_c | t_c
 __device__ __forceinline__ void k2c_stream_map(const double* s_cam, int c, const double (&pose)[6], double (&Rc)[9],
@@ -500,7 +410,7 @@ __global__ void __launch_bounds__(kW * 32, 1) k2c_pose_kernel(const K2CParams p)
       const int c = __ffs(m) - 1;
       double Rc[9], K[9];
       k2c_stream_map(s.cam, c, pose, Rc, K);
-      k2c_mbar_wait(s.bar + (k_c & 1u), (k_c >> 1) & 1u);
+      mbar_wait(s.bar + (k_c & 1u), (k_c >> 1) & 1u);
       pose_block_add(s.ring + (size_t)(k_c & 1u) * kStreamStage + lane - 36 * kTile, Rc, K, Vpp, gpp);   // stage row 0 = hand-off row 36
       __syncwarp();
       asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
@@ -562,12 +472,15 @@ __global__ void __launch_bounds__(kW * 32, 1) k2c_rows_kernel(const K2CParams p)
     if (it_i >= n_it) return;
     if (sub_i == 0) tile_i = unit_of(gw + (long long)it_i * nW, c_i);
     if (lane == 0) {
-      const unsigned b = k2c_smem_u32(s.bar + (k_i & 1u));
+      // the barrier's shared address is converted once, ahead of the stage addresses, and serves the expect_tx and
+      // every copy of the stage: spelt with mbar_expect_tx / tma_load_1d, the conversion moves into each call and
+      // ptxas schedules this issue path differently
+      const unsigned b = smem_u32(s.bar + (k_i & 1u));
       double* st = s.ring + (size_t)(k_i & 1u) * kStreamStage;
       const double* hp = p.H + (size_t)(tile_i * C + c_i) * kHandoff * kTile;
       auto copy = [&](double* dst, const double* src, unsigned rows) {
         asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                         k2c_smem_u32(dst)),
+                         smem_u32(dst)),
                      "l"(src), "r"(rows * kTile * (unsigned)sizeof(double)), "r"(b)
                      : "memory");
       };
@@ -588,7 +501,7 @@ __global__ void __launch_bounds__(kW * 32, 1) k2c_rows_kernel(const K2CParams p)
   };
   unsigned k_c = 0;
   auto acquire = [&]() -> const double* {
-    k2c_mbar_wait(s.bar + (k_c & 1u), (k_c >> 1) & 1u);
+    mbar_wait(s.bar + (k_c & 1u), (k_c >> 1) & 1u);
     return s.ring + (size_t)(k_c & 1u) * kStreamStage + lane;
   };
   auto release = [&]() {
@@ -699,27 +612,22 @@ __global__ void __launch_bounds__(256) k2c_grad_kernel(const K2CParams p) {
 }
 
 // ------------------------------------------------------------------ launchers
-// K2c variant and the number of per-CTA partial outputs (Z y, max |g|) it produces.
-// K2c variant (0 general, 1 staged ring, 2 streamed) and the number of per-CTA partial outputs (Z y, max |g|)
-// it produces: 0 general, 1 staged ring, 2 streamed pair.
-// MCBA_K2C_MODE = general | ring | stream overrides the choice (A/B runs, debugging).
 int k2c_stream_warps(int C) {
   int w = 12;
   while (w > 1 && k2c_stream_smem(C, w) > 227u * 1024u) --w;
   return w >= 12 ? 12 : (w >= 10 ? 10 : (w >= 8 ? 8 : 4));
 }
+// K2c variant (1 staged ring, 2 streamed pair) and the number of per-CTA partial outputs (Z y, max |g|) it produces.
 int k2_consumer_parts(const Layout& L, int n_sm, int* mode) {
-  static const char* forced = getenv("MCBA_K2C_MODE");
-  static const bool no_ring = getenv("MCBA_K2C_GENERAL") != nullptr;   // older switch: force the general path
   // measured on B200: the staged ring wins where it applies (6 x 50,000: 0.076 ms against 0.023 + 0.050 ms for the
   // streamed pair, and clearly on small shards, where one tile per warp leaves most warps of the pose kernel idle);
-  // the streamed pair replaces the general path for more cameras (16 x 25,000: 0.146 -> 0.114 ms)
-  int m = L.C >= 2 && L.C <= 6 ? 1 : 2;
-  if (no_ring) m = 0;
-  if (forced) m = forced[0] == 's' ? 2 : (forced[0] == 'r' && L.C >= 2 && L.C <= 6 ? 1 : 0);
-  *mode = m;
-  if (m == 2) return (int)(L.nTiles < n_sm ? L.nTiles : n_sm);
-  return m == 1 ? (int)(L.nTiles < 2 * n_sm ? L.nTiles : 2 * n_sm) : (int)L.nTiles;
+  // the streamed pair serves every other camera count (16 x 25,000: 0.114 ms against 0.146 ms for one CTA per tile)
+  if (L.C >= 2 && L.C <= 6) {
+    *mode = 1;
+    return (int)(L.nTiles < 2 * n_sm ? L.nTiles : 2 * n_sm);
+  }
+  *mode = 2;
+  return (int)(L.nTiles < n_sm ? L.nTiles : n_sm);
 }
 
 int k2_producer_grid(const Layout& L, int n_sm, int* warps) {
@@ -838,7 +746,7 @@ int launch_k2_consumer(mcba_handle* h, const double* x, double lambda) {
       default: MCBA_K2C_STREAM(4); break;
     }
 #undef MCBA_K2C_STREAM
-  } else if (h->k2c_mode == 1) {
+  } else {
     const int C = L.C;
     const size_t smem = sizeof(double) * ((size_t)C * kHandoff * kTile + (size_t)C * kXchg * kTile);
     const int grid = h->n_part_c;
@@ -855,11 +763,6 @@ int launch_k2_consumer(mcba_handle* h, const double* x, double lambda) {
       default: MCBA_K2C_RING(6); break;
     }
 #undef MCBA_K2C_RING
-  } else {
-    const int grid = (int)L.nTiles;
-    if (L.C >= 6) k2c_kernel<6><<<grid, 192, 0, h->stream>>>(p);
-    else if (L.C >= 3) k2c_kernel<3><<<grid, 96, 0, h->stream>>>(p);
-    else k2c_kernel<1><<<grid, 32, 0, h->stream>>>(p);
   }
   h->launches++;
   MCBA_CUDA(cudaGetLastError());

@@ -25,44 +25,10 @@ __host__ __device__ inline int tile_index(int bi, int bj, int nb) { return bi * 
 // mapping (lane -> row I*8 + lane/4, k = k0 + lane%4), so one load serves both roles.
 // B200: DMMA and DFMA share the FP64 pipe at the same FMA rate (profiles/r01_b_ubench_*), but
 // one DMMA replaces 8 DFMA issue slots and all the operand shuffling of a register-tiled SYRK.
-__device__ __forceinline__ unsigned smem_u32(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
-
-__device__ __forceinline__ void mbar_init(unsigned long long* bar, unsigned count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(unsigned long long* bar, unsigned bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(unsigned long long* bar, unsigned parity) {
-  asm volatile(
-      "{\n"
-      ".reg .pred p;\n"
-      "WAIT_LOOP:\n"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-      "@p bra WAIT_DONE;\n"
-      "bra WAIT_LOOP;\n"
-      "WAIT_DONE:\n"
-      "}\n" ::"r"(smem_u32(bar)), "r"(parity) : "memory");
-}
-__device__ __forceinline__ void tma_load_1d(void* dst, const void* src, unsigned bytes, unsigned long long* bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(smem_u32(dst)),
-               "l"(src), "r"(bytes), "r"(smem_u32(bar))
-               : "memory");
-}
-__device__ __forceinline__ void dmma_m8n8k4(double& c0, double& c1, double a, double b) {
-  asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};"
-               : "+d"(c0), "+d"(c1)
-               : "d"(a), "d"(b));
-}
-
 constexpr int kSyrkStages = 3;
 // consumer (DMMA) warps kW = 8 (<= 96 tiles: 6 cameras) or 15 (up to 300 tiles: 16 cameras without
 // re-reading Z; 15 + 1 warps = 4 per scheduler leaves 128 registers per thread); warp kW is the copy producer
 constexpr int kZK = 6 * kTile;    // K extent of one tile of Z
-
-__device__ __forceinline__ void mbar_arrive(unsigned long long* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
 
 struct SyrkParams {
   const double* Z;

@@ -43,12 +43,6 @@ constexpr int kSolveMaxN = 192;   // 16 cameras; larger systems take the library
 
 __host__ __device__ __forceinline__ int pk(int i, int j) { return i * (i + 1) / 2 + j; }   // j <= i
 
-__device__ __forceinline__ void solve_dmma(double& c0, double& c1, double a, double b) {
-  asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};"
-               : "+d"(c0), "+d"(c1)
-               : "d"(a), "d"(b));
-}
-
 // 1/sqrt(t), t > 0 in the normal range: MUFU.RSQ64H seed (> 20 bits) and ONE third-order correction
 // (relative error ~ (5/16) e^3 < 2^-60); four dependent FP64 operations instead of the library's
 // slow path on the critical chain of every pivot.  Non-positive or NaN t gives NaN / inf, which the
@@ -76,8 +70,9 @@ struct SolveParams {
 // panel's 8 x 8 block do not fit in 128 registers (they spilled to local memory: 0.116 ms for 192 x 192), so that
 // variant keeps the tiles where they already live -- the packed matrix in shared memory -- and every update is
 // load, two DMMAs, store; the 19 tiles of a warp are independent, so their round trips overlap.
-template <int kT, bool kSmemAcc = false>
+template <int kT>
 __global__ void __launch_bounds__(kSolveThreads, 1) solve_reduced_kernel(const SolveParams p) {
+  constexpr bool kSmemAcc = kT > 8;
   extern __shared__ double A[];                 // packed lower triangle of the augmented matrix, n1p rows
   __shared__ double s_inv[kSolveMaxN + 8];      // 1 / L_jj
   __shared__ int s_info;
@@ -228,13 +223,13 @@ __global__ void __launch_bounds__(kSolveThreads, 1) solve_reduced_kernel(const S
         const int cr = ib * 8 + fr, cc = jb * 8 + fc;
         if (kSmemAcc) {                 // the tile lives in shared memory (fragments read the panel's columns only)
           double c0 = cc <= cr ? A[pk(cr, cc)] : 0.0, c1 = cc + 1 <= cr ? A[pk(cr, cc + 1)] : 0.0;
-          solve_dmma(c0, c1, a0, b0);
-          solve_dmma(c0, c1, a1, b1);
+          dmma_m8n8k4(c0, c1, a0, b0);
+          dmma_m8n8k4(c0, c1, a1, b1);
           if (cc <= cr) A[pk(cr, cc)] = c0;
           if (cc + 1 <= cr) A[pk(cr, cc + 1)] = c1;
         } else {
-          solve_dmma(acc[s][0], acc[s][1], a0, b0);
-          solve_dmma(acc[s][0], acc[s][1], a1, b1);
+          dmma_m8n8k4(acc[s][0], acc[s][1], a0, b0);
+          dmma_m8n8k4(acc[s][0], acc[s][1], a1, b1);
           if (jb == kb + 1) {           // the next panel: back to shared memory
             if (cc <= cr) A[pk(cr, cc)] = acc[s][0];
             if (cc + 1 <= cr) A[pk(cr, cc + 1)] = acc[s][1];
@@ -306,10 +301,9 @@ int solve_tier(int nc) {
   if (solve_uses_library(nc)) return kSolveTierLibrary;
   const int n1p = (nc + 1 + 7) & ~7;
   const int nb = n1p / 8, per_warp = ((nb - 1) * nb / 2 + kSolveWarps - 1) / kSolveWarps;
-  static const bool wide_in_registers = getenv("MCBA_SOLVE_WIDE_REGS") != nullptr;   // A/B: the spilling variant
   if (per_warp <= 3) return kSolveTierRegs3;
   if (per_warp <= 8) return kSolveTierRegs8;
-  return wide_in_registers ? kSolveTierRegs19 : kSolveTierSmem19;
+  return kSolveTierSmem19;
 }
 
 // cuSOLVER handle on the handle's stream and the potrf workspace of the 12C-wide solve, created on first use
@@ -338,15 +332,14 @@ int solve_reduced(mcba_handle* h, double lambda) {
     p.D2cam = h->d_D2cam; p.dcam = h->d_dcam; p.info = h->d_info; p.fixed = h->any_fixed ? h->d_fixed : nullptr;
     const int n1p = (nc + 1 + 7) & ~7;
     const size_t smem = sizeof(double) * (size_t)n1p * (n1p + 1) / 2;
-#define MCBA_SOLVE(...)                                                                                                    \
+#define MCBA_SOLVE(KT)                                                                                                     \
   do {                                                                                                                     \
-    MCBA_CUDA(set_dynamic_smem((const void*)solve_reduced_kernel<__VA_ARGS__>, smem)); \
-    solve_reduced_kernel<__VA_ARGS__><<<1, kSolveThreads, smem, h->stream>>>(p);                                           \
+    MCBA_CUDA(set_dynamic_smem((const void*)solve_reduced_kernel<KT>, smem));                                              \
+    solve_reduced_kernel<KT><<<1, kSolveThreads, smem, h->stream>>>(p);                                                    \
   } while (0)
     if (tier == kSolveTierRegs3) MCBA_SOLVE(3);
     else if (tier == kSolveTierRegs8) MCBA_SOLVE(8);
-    else if (tier == kSolveTierRegs19) MCBA_SOLVE(19);
-    else MCBA_SOLVE(19, true);
+    else MCBA_SOLVE(19);
 #undef MCBA_SOLVE
 #ifdef MCBA_SOLVE_TIMING
     {

@@ -121,20 +121,18 @@ static int evaluate(mcba_handle* h, const double* x, double lambda, int loss, do
 }
 
 // K2c + SYRK + finalize (+ all-reduce) on the K2p outputs the handle currently points at.
-// need_system = false: the evaluation that closes a solve only has to deliver the gradient, b and the
-// scalars at the final point -- the SYRK (sum Z Z^T, a fifth of an evaluation) is skipped and the S
-// part of d_red is left stale (nothing reads it before the next evaluation rebuilds it).
+// need_system = false: the evaluation that closes a solve only has to deliver the gradient and the
+// scalars at the final point -- K2c and the SYRK are skipped.
 static int evaluate_tail(mcba_handle* h, const double* x, double lambda, bool need_system = true) {
   int rc;
-  static const bool full_closing = getenv("MCBA_FULL_CLOSING_EVAL") != nullptr;   // A/B: K2c instead of the gradient kernel
-  if (!need_system && !full_closing) {
+  if (!need_system) {
     // gradient and cost only: the pose gradients come from a kernel that reads just the q_ext rows of the hand-off
     // (no Z, no factor: b and S in d_red are left stale, nothing reads them before the next evaluation rebuilds them)
     if ((rc = launch_k2_gradient(h, x))) return rc;
     return finalize_and_sum(h);
   }
   if ((rc = launch_k2_consumer(h, x, lambda))) return rc;
-  if (need_system && (rc = launch_k2_syrk(h))) return rc;
+  if ((rc = launch_k2_syrk(h))) return rc;
   return finalize_and_sum(h);
 }
 
@@ -357,7 +355,7 @@ static int create_impl(mcba_handle* h, int C, int64_t F, int N, int device) {
   MCBA_ALLOC(h->d_active, L.nTiles);
   MCBA_ALLOC(h->d_units, (size_t)C * L.nTiles);
   MCBA_ALLOC(h->d_unit_count, 128);
-  MCBA_ALLOC(h->d_row_off, std::max(((size_t)C * F * N + 31) / 32, (size_t)C * ((F + 31) / 32)) + 1);
+  MCBA_ALLOC(h->d_row_off, (size_t)C * ((F + 31) / 32) + 1);
   MCBA_ALLOC(h->d_x, n);
   MCBA_ALLOC(h->d_xtrial, n);
   MCBA_ALLOC(h->d_cams, C);
@@ -433,7 +431,7 @@ int mcba_destroy(mcba_handle* h) {
   if (h->peer_block) cudaFree(h->peer_block);
   void* ptrs[] = {h->d_obs_ref, h->d_obs_tiled, h->d_obj, h->d_row_off, h->d_x, h->d_xtrial, h->d_cams, h->d_Z,
                   h->d_Linv, h->d_y, h->d_JlTau, h->d_gpose, h->d_D2pose, h->d_D2cam, h->d_partU, h->d_partS, h->d_partSyrk,
-                  h->d_red, h->d_Sd, h->d_dcam, h->d_scal, h->d_info, h->d_work, h->d_Sraw, h->d_H, h->d_H_alt, h->d_partU_alt, h->d_partS_alt, h->d_cams_alt, h->d_partG, h->d_partZy, h->d_perm, h->d_mask, h->d_active, h->d_sort_tmp, h->d_units, h->d_unit_count, h->d_rowT, h->d_chunk_rows, h->d_fin_scratch, h->d_fin_counter, h->d_fixed};
+                  h->d_red, h->d_Sd, h->d_dcam, h->d_scal, h->d_info, h->d_work, h->d_Sraw, h->d_H, h->d_H_alt, h->d_partU_alt, h->d_partS_alt, h->d_cams_alt, h->d_partG, h->d_partZy, h->d_perm, h->d_mask, h->d_active, h->d_sort_tmp, h->d_units, h->d_unit_count, h->d_chunk_rows, h->d_fin_scratch, h->d_fin_counter, h->d_fixed};
   for (void* p : ptrs) if (p) cudaFree(p);
   if (h->prof_ev) {
     for (int i = 0; i < kProfEvents * kProfRing; ++i) cudaEventDestroy(h->prof_ev[i]);

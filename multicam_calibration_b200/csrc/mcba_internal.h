@@ -63,9 +63,8 @@ struct mcba_handle {
   int* d_unit_count = nullptr;       // [0..C) live units per camera | [32..32+C] group prefix for K2p | [96..97] finite scalars (u64, K2p's count)
   void* d_sort_tmp = nullptr;
   size_t sort_tmp_bytes = 0;
-  long long* d_row_off = nullptr;  // exclusive scan of finite scalars per group of 32 (c,f,n) slots
+  long long* d_row_off = nullptr;  // [C * nBlk + 1] exclusive scan of finite scalars per K1 chunk
   unsigned int* d_chunk_rows = nullptr;   // [C * nBlk] per K1 chunk: rows (camera, frame) with at least one finite scalar (lazy)
-  double* d_rowT = nullptr;        // [C*F][12] composed (camera o pose) transforms, K1 only (lazy)
   long long m = 0;                 // finite scalar residuals
   long long n_obs = 0;             // (c,f,n) with at least one finite scalar
   bool have_obs = false;
@@ -114,8 +113,8 @@ struct mcba_handle {
   unsigned long long* d_signal_flag = nullptr;
   unsigned long long signal_seq = 0;
   cudaEvent_t readback_done = nullptr;
-  int n_part_c = 0;           // K2c partial outputs (one per tile, or one per persistent CTA on the ring path)
-  int k2c_mode = 0;           // 0 general, 1 staged ring (2..6 cameras), 2 streamed pair (k2_frames.cu)
+  int n_part_c = 0;           // K2c partial outputs (one per persistent CTA)
+  int k2c_mode = 0;           // 1 staged ring (2..6 cameras), 2 streamed pair (any other count; k2_frames.cu)
   int grid_frames = 0, prod_warps = 8, grid_syrk = 0, grid_cost = 0, grid_back = 0;
   // solver
   cusolverDnHandle_t solver = nullptr;
@@ -191,7 +190,7 @@ int k2c_stream_warps(int C);
 // SYRK CTA width (warps), CTA rows (gy) and the block count of the compiled tile list (0: run-time list)
 void syrk_plan(int nc, int* warps, int* gy, int* static_nb);
 // solve of the reduced system: tiles per warp of the one-CTA kernel, or the library
-enum SolveTier : int { kSolveTierLibrary = 0, kSolveTierRegs3 = 3, kSolveTierRegs8 = 8, kSolveTierRegs19 = 19, kSolveTierSmem19 = 119 };
+enum SolveTier : int { kSolveTierLibrary = 0, kSolveTierRegs3 = 3, kSolveTierRegs8 = 8, kSolveTierSmem19 = 119 };
 int solve_tier(int nc);
 // dynamic shared memory of the observation transpose (k1_residual.cu): [32 frames][N + 1] corners
 inline size_t tile_observations_smem(int N) { return sizeof(double2) * kTile * ((size_t)N + 1); }

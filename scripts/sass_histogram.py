@@ -14,7 +14,7 @@ import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 LIB = os.path.join(ROOT, "multicam_calibration_b200", "libmcba.so")
-HOT = ["k2p_kernel", "k2c_ring_kernel", "k2c_pose_kernel", "k2c_rows_kernel", "k2c_kernel", "sum_children_kernel", "k2_syrk_kernel", "finalize_kernel", "solve_reduced_kernel",
+HOT = ["k2p_kernel", "k2c_ring_kernel", "k2c_pose_kernel", "k2c_rows_kernel", "sum_children_kernel", "k2_syrk_kernel", "finalize_kernel", "solve_reduced_kernel",
        "backsub_kernel", "sum_scalars_kernel", "peer_allreduce_kernel", "residual_chunks_kernel", "cost_kernel",
        "triangulate_kernel", "project_points_multi_kernel", "homography_transfer_kernel", "tile_observations_kernel",
        "frame_errors_kernel"]

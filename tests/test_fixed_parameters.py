@@ -200,7 +200,6 @@ TIERS = {
     "6x50000": (lambda: _scene(6, 50000), "regs3", None),
     "10x8000": (lambda: _scene(10, 8000, seed=11), "regs8", None),
     "16x8000": (lambda: _scene(16, 8000, seed=16), "smem19", None),
-    "16x8000_wide_regs": (lambda: _scene(16, 8000, seed=16), "regs19", {"MCBA_SOLVE_WIDE_REGS": "1"}),
     "6x8000_cusolver": (lambda: _scene(6, 8000, seed=1), "cusolver", {"MCBA_CUSOLVER": "1"}),
     "20x2000": (lambda: _scene(20, 2000, seed=20), "cusolver", None),
 }

@@ -187,9 +187,9 @@ def test_many_cameras_reduced_system_matches_oracle():
 
 @pytest.mark.parametrize("C,F", [(1, 40), (2, 31), (3, 65), (5, 33), (7, 96), (12, 40)])
 def test_camera_count_sweep_step_and_solve(C, F):
-    """Every camera count takes its own variants of K2c (ring <= 6 cameras / general), of the SYRK tile
+    """Every camera count takes its own variants of K2c (ring 2-6 cameras / streamed), of the SYRK tile
     lists, of the finalize grid and of the solve kernel (12 C not a multiple of 8: partial last panel;
-    3 / 8 / 19 register tiles per warp): reduced system and damped step against the dense oracle, then
+    3 / 8 register tiles per warp, 19 in shared memory): reduced system and damped step against the dense oracle, then
     the LM loop down to the oracle's own minimum."""
     sc = make_scene(C, F, sigma=0.3, p_missing_view=0.25 if C > 2 else 0.0, p_missing_corner=0.05, seed=40 + C)
     x0 = sc.x0()
