@@ -54,7 +54,9 @@ def reprojection_residuals(all_calib_uvs, all_extrinsics, all_intrinsics, calib_
     C, F, N, _ = uvs.shape
     if poses.shape[0] != F or obj.shape != (N, 3) or len(all_extrinsics) != C or len(all_intrinsics) != C:
         raise ValueError("reprojection_residuals: inconsistent shapes")
-    ext = np.ascontiguousarray(np.stack([np.asarray(e, dtype=np.float64) for e in all_extrinsics]))
+    if F == 0:   # no frame, no distance: empty outputs and NaN medians (empty tensors have no device pointer)
+        return np.full(C, np.nan), np.zeros((C, 0, N, 2)), np.zeros((C, 0, N, 2))
+    ext =np.ascontiguousarray(np.stack([np.asarray(e, dtype=np.float64) for e in all_extrinsics]))
     Ks = np.ascontiguousarray(np.stack([np.asarray(K, dtype=np.float64) for K, _ in all_intrinsics]))
     dist = np.zeros((C, 5))
     for c, (_, d) in enumerate(all_intrinsics):

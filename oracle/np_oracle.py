@@ -651,7 +651,7 @@ def lm_solve(x0, all_calib_uvs, calib_objpoints, ftol=1e-4, xtol=1e-8, gtol=1e-8
 FLT_EPS = float(np.finfo(np.float32).eps)
 
 
-def homography_dlt(src, dst):
+def homography_dlt(src, dst, round32=True):
     """First half of ``cv2.findHomography(src, dst)`` with ``method=0`` (viz.py:166).
 
     OpenCV is an un-vendored binary dependency (4.13.0 in the build container); this restates the
@@ -660,10 +660,12 @@ def homography_dlt(src, dst):
     normal matrix of the DLT rows ``[X Y 1 0 0 0 -xX -xY -x]`` / ``[0 0 0 X Y 1 -yX -yY -y]`` is
     accumulated and its eigenvector of the smallest eigenvalue, de-normalised and divided by
     ``H[2,2]``, is the estimate.  Returns ``(H0, src32, dst32)`` (the rounded points as float64).
-    Pinned numerically against cv2 through ``tests/golden/qc.npz``.
+    Pinned numerically against cv2 through ``tests/golden/qc.npz``.  ``round32=False`` skips the
+    float32 conversion (not what OpenCV does; the tests use it as a wrong kernel).
     """
-    M = np.asarray(src, dtype=np.float32).astype(np.float64)
-    m = np.asarray(dst, dtype=np.float32).astype(np.float64)
+    t = np.float32 if round32 else np.float64
+    M = np.asarray(src, dtype=t).astype(np.float64)
+    m = np.asarray(dst, dtype=t).astype(np.float64)
     n = len(M)
     cM, cm = M.sum(0) / n, m.sum(0) / n
     sM, sm = n / np.abs(M - cM).sum(0), n / np.abs(m - cm).sum(0)
