@@ -1167,11 +1167,12 @@ int mcba_lm_run(mcba_handle* h, double* d_x, const mcba_options* opt_in, mcba_re
       // same point, same cost and gradient: nothing to read back
     }
   }
-  if (pending) {   // left the loop (budget / xtol) with an evaluation still in flight
+  if (pending) {   // left the loop on the evaluation budget with the last accepted point's scalars in flight
+    // (a step that met ftol / xtol was settled at once, a rejection settles before it is decided): settle them
+    // now, so that gtol met at that point reports status 1 rather than 0 -- scipy's trf tests gtol before the
+    // budget, and so does every rank, since gnorm is the all-reduced maximum
     MCBA_CUDA(cudaStreamSynchronize(h->stream));
-    const int keep = status;
     settle();
-    status = keep;
   }
 
   MCBA_CUDA(cudaMemcpyAsync(d_x, x, sizeof(double) * n_local, cudaMemcpyDeviceToDevice, h->stream));
